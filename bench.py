@@ -2,6 +2,7 @@
 """Benchmark of the reconcile tick — BASELINE.json's metric on its config.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload C3|C3-steady|C2|C5|C4]
+                    [--dump-outputs DIR]
 
 metric   pod-group reconciles/sec: pod groups brought up to date / time of one tick (fused pod
          scan + group pass, LWS pass; the placement round when the workload has
@@ -67,7 +68,13 @@ def parse():
                     help="replay CUDA graphs instead of eager launches (measured slower: programmatic "
                          "dependent launch does not span graph replays)")
     ap.add_argument("--no-check", action="store_true", help="skip the oracle comparison of the outputs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the result tables of the last one (rank 0's) as DIR/<table>.npy; "
+                         "the inputs are seeded, so two builds run with the same arguments can be compared table by table")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def measured_peak():
@@ -128,6 +135,28 @@ class ClockSampler:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": [], "samples": 0}
         return {"sm_mhz": float(np.median(sm)), "sm_max_mhz": float(max(mx)), "reasons": sorted(reasons),
                 "samples": len(sm)}
+
+
+DUMP_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(out_dir, tables):
+    """Write each result table as <out_dir>/<name>.npy: float64, one row per record, one column per
+    field in record order (every field is a 32-bit integer, so float64 holds it exactly).  Should the
+    tables exceed DUMP_BYTES in all, each keeps the same share of its rows, drawn with a fixed seed,
+    and <name>_rows.npy lists which."""
+    arrays = {name: (np.stack([a[f] for f in a.dtype.names], axis=1) if a.dtype.names else a).astype(np.float64)
+              for name, a in tables.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    share = 1.0 if total <= DUMP_BYTES else DUMP_BYTES / (2 * total)  # the row indices cost at most as much again
+    rng = np.random.default_rng(0)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if share < 1.0:
+            rows = np.sort(rng.choice(len(a), int(len(a) * share), replace=False))
+            a = a[rows]
+            np.save(os.path.join(out_dir, f"{name}_rows.npy"), rows.astype(np.float64))
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def host_threads() -> int:
@@ -270,6 +299,11 @@ def run_reference(args):
         i += 1
     dt = time.perf_counter() - t0
     value = len(t.groups) * args.steps / dt
+    if args.dump_outputs:
+        outs = {"lws_out": arm.lws_out, "group_out": arm.group_out}
+        if arm.place_out is not None:
+            outs["place_out"] = arm.place_out
+        dump_outputs(args.dump_outputs, outs)
     # the same arm sweeping everything every step (no event source): reported beside it
     full = CpuArm(t, threads)
     full.full_step()
@@ -307,9 +341,11 @@ def run_reference_ds(args):
     oracle.sweep_ds(d.ds, d.roles, d.revroles)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        oracle.sweep_ds(d.ds, d.roles, d.revroles)
+        outs = oracle.sweep_ds(d.ds, d.roles, d.revroles)
     dt = time.perf_counter() - t0
     value = n_ds * args.steps / dt
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(("ds_out", "ds_role_out", "ds_revrole_out"), outs)))
     print(json.dumps({
         "impl": "reference", "metric": "DisaggregatedSet reconciles/sec (2-role rollout partition calc)", "value": value,
         "unit": "sets/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -381,6 +417,11 @@ def run_ours_ds(args):
         barrier()
         ms = e0.elapsed_time(e1) / args.steps
         launches = eng.launch_count - l0
+        if args.dump_outputs and rank == 0:
+            last = sets[(args.steps - 1) % copies]
+            dump_outputs(args.dump_outputs, {"ds_out": last["o1"].cpu().numpy().view(R.DS_OUT),
+                                             "ds_role_out": last["o2"].cpu().numpy().view(R.DS_ROLE_OUT),
+                                             "ds_revrole_out": last["o3"].cpu().numpy().view(R.DS_REVROLE_OUT)})
         for i in range(20000):
             step(i)
         torch.cuda.synchronize()
@@ -628,6 +669,13 @@ def run_ours(args):
     with ClockSampler(local_rank) as clk:
         ms_step, launches = timed(full_step, args.steps, W)
         host_ms_step = getattr(timed, "host_ms", None)
+        if args.dump_outputs and rank == 0:  # before the passes below write into the same buffers
+            last = sets[(args.steps - 1) % copies]
+            outs = {"lws_out": last["lo"].cpu().numpy().view(R.LWS_OUT),
+                    "group_out": last["go"].cpu().numpy().view(R.GROUP_OUT)}
+            if place_on and n_req:
+                outs["place_out"] = d_pout.cpu().numpy()[: n_req * R.PLACE_OUT.itemsize].view(R.PLACE_OUT)
+            dump_outputs(args.dump_outputs, outs)
         # each pass alone (same rotating inputs), for the per-kernel roofline
         ms_sweep, _ = timed(lambda i: sweep(i, t.flags), args.steps, 3)
         ms_fused, _ = timed(lambda i: sweep(i, t.flags | R.SWEEP_SKIP_LWS_PASS), args.steps, 3)

@@ -1,11 +1,27 @@
 """The bench.py JSON line: the committed N=1 line of this round (profiles/r2_bench_line_n1.json) has
-every key the contract names, and the reference arm — which runs on CPU — still prints its line."""
+every key the contract names, and the reference arm — which runs on CPU — still prints its line.
+--dump-outputs writes what the timed path computed in its last step."""
 import json
 import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
+
+def run_bench(*args, timeout=600):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args], capture_output=True, text=True,
+                       timeout=timeout)
+    assert r.returncode == 0, r.stderr[-2000:]
+    return json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1])
+
+
+def columns(records):
+    """A record table as --dump-outputs writes it: float64, one column per field."""
+    return np.stack([records[f] for f in records.dtype.names], axis=1).astype(np.float64)
 
 
 def test_committed_bench_line_has_the_contract_keys():
@@ -36,9 +52,39 @@ def test_committed_bench_line_has_the_contract_keys():
 
 
 def test_reference_arm_prints_its_line_on_cpu():
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--workload", "C2",
-                        "--steps", "2", "--warmup", "1"], capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stderr[-2000:]
-    line = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1])
+    line = run_bench("--impl", "reference", "--workload", "C2", "--steps", "2", "--warmup", "1")
     assert line["impl"] == "reference" and line["unit"] == "groups/s" and line["value"] > 0
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["cpu_baseline"]["kind"] in ("port", "reference")
+
+
+def test_reference_arm_dumps_its_last_step(tmp_path):
+    """--dump-outputs writes the result tables of the last timed step, one float64 column per record
+    field; the inputs are seeded, so a second run writes the same arrays."""
+    from lws_b200 import records as R
+
+    args = ("--impl", "reference", "--workload", "C2", "--steps", "2", "--warmup", "1", "--dump-outputs")
+    line = run_bench(*args, str(tmp_path / "a"))
+    run_bench(*args, str(tmp_path / "b"))
+    for name, dt, rows in (("lws_out", R.LWS_OUT, line["config"]["lws"]), ("group_out", R.GROUP_OUT, line["config"]["groups"])):
+        a, b = np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy")
+        assert a.dtype == np.float64 and a.shape == (rows, len(dt.names)), name
+        assert np.array_equal(a, b), name
+
+
+@pytest.mark.gpu
+def test_dumped_outputs_are_the_tick_results(tmp_path):
+    """--dump-outputs on the engine: the tables of the last timed tick equal the CPU oracle's on the
+    same seeded cluster."""
+    import oracle
+    from lws_b200 import records as R
+    from lws_b200 import synth
+
+    run_bench("--workload", "C3", "--scale", "0.1", "--steps", "3", "--warmup", "1", "--e2e-steps", "10",
+              "--dump-outputs", str(tmp_path), timeout=900)
+    t = synth.make("C3", 0.1, seed=synth.SEED)
+    reqs = t.place_requests()
+    assert len(reqs) > 0
+    lo, go, _ = oracle.sweep_lws(t.lws, t.groups, t.pod_state, t.pod_ident, t.nodes, flags=t.flags)
+    po = oracle.place(t.nodes, R.occupancy_of(t.pod_ident, len(t.nodes)), t.n_domains, t.n_namespaces, reqs)
+    for name, want in (("lws_out", lo), ("group_out", go), ("place_out", po)):
+        assert np.array_equal(np.load(tmp_path / f"{name}.npy"), columns(want)), name
