@@ -117,6 +117,49 @@ func (e *Engine) Place(reqs *C.lwse_place_req, n uint32, occupancy *C.uint32_t, 
 // SweepDs advances every DisaggregatedSet by one reconcile.
 func (e *Engine) SweepDs(t *C.lwse_ds_tables) error { return e.check(C.lwse_sweep_ds_host(e.h, t)) }
 
+// DsResidentLoad copies the three DisaggregatedSet input tables to the device, where they stay
+// (their own buffers: SweepDs and the LWS resident tables never touch them).  Committed results
+// start at zero; the next DsTick lists every owned row.
+func (e *Engine) DsResidentLoad(t *C.lwse_ds_tables) error { return e.check(C.lwse_ds_resident_load(e.h, t)) }
+
+// DsTickResult: views of engine-owned pinned memory, valid until the next resident call.
+type DsTickResult struct {
+	DsRows      []uint32
+	DsOut       []C.lwse_ds_out
+	RoleRows    []uint32
+	RoleOut     []C.lwse_ds_role_out
+	RevroleRows []uint32
+	RevroleOut  []C.lwse_ds_revrole_out
+}
+
+// DsTick is one pass of the DS controller's work queue (lwse_ds_resident_tick): the patch segments
+// (tables LWSE_TABLE_DS .. LWSE_TABLE_DS_REVROLES, ideally in the arena) in, the listed rows out —
+// the DS keys that need work with their current ds_out, and their role / (revision, role) rows
+// whose decision changed.  Still uncompiled, like the rest of this file.
+func (e *Engine) DsTick(segs []C.lwse_patch_seg) (DsTickResult, error) {
+	var t C.lwse_ds_tick
+	if len(segs) > 0 {
+		t.segs = &segs[0]
+		t.n_segs = C.uint32_t(len(segs))
+	}
+	if err := e.check(C.lwse_ds_resident_tick(e.h, &t)); err != nil {
+		return DsTickResult{}, err
+	}
+	return DsTickResult{
+		DsRows:      unsafe.Slice((*uint32)(unsafe.Pointer(t.ds_rows)), int(t.n_ds)),
+		DsOut:       unsafe.Slice(t.ds_out, int(t.n_ds)),
+		RoleRows:    unsafe.Slice((*uint32)(unsafe.Pointer(t.role_rows)), int(t.n_roles)),
+		RoleOut:     unsafe.Slice(t.role_out, int(t.n_roles)),
+		RevroleRows: unsafe.Slice((*uint32)(unsafe.Pointer(t.revrole_rows)), int(t.n_revroles)),
+		RevroleOut:  unsafe.Slice(t.revrole_out, int(t.n_revroles)),
+	}, nil
+}
+
+// DsResidentOutputs copies every committed DS result row into the caller's tables (nil skips one).
+func (e *Engine) DsResidentOutputs(ds *C.lwse_ds_out, roles *C.lwse_ds_role_out, revroles *C.lwse_ds_revrole_out) error {
+	return e.check(C.lwse_ds_resident_outputs(e.h, ds, roles, revroles))
+}
+
 // GroupKeys computes SHA-1 digests (20 bytes each) of n strings laid out CSR-style.
 func (e *Engine) GroupKeys(bytes *C.uint8_t, offsets *C.uint32_t, n uint32, digests *C.uint8_t) error {
 	return e.check(C.lwse_group_keys_host(e.h, bytes, offsets, C.uint32_t(n), digests))

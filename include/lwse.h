@@ -370,7 +370,10 @@ typedef enum lwse_table {
   LWSE_TABLE_GROUPS = 1,    /* lwse_group_rec  */
   LWSE_TABLE_POD_STATE = 2, /* lwse_pod_state  */
   LWSE_TABLE_POD_IDENT = 3, /* lwse_pod_ident  */
-  LWSE_TABLE_PLACE_REQS = 4 /* lwse_place_req (lwse_resident_place_load)  */
+  LWSE_TABLE_PLACE_REQS = 4, /* lwse_place_req (lwse_resident_place_load)  */
+  LWSE_TABLE_DS = 5,          /* lwse_ds_rec          (lwse_ds_resident_tick only) */
+  LWSE_TABLE_DS_ROLES = 6,    /* lwse_ds_role_rec     (lwse_ds_resident_tick only) */
+  LWSE_TABLE_DS_REVROLES = 7  /* lwse_ds_revrole_rec  (lwse_ds_resident_tick only) */
 } lwse_table;
 
 /* Result rows that differ from the previous resident sweep (all rows after a load).
@@ -706,6 +709,58 @@ typedef struct lwse_ds_tables {
 
 LWSE_API int lwse_sweep_ds_host(lwse_engine* e, const lwse_ds_tables* host_tables);
 LWSE_API int lwse_sweep_ds_device(lwse_engine* e, const lwse_ds_tables* dev_tables, void* stream);
+
+/* ---- the resident DS tick: what one pass of the DisaggregatedSet controller's work queue maps to --
+ * The three DS input tables stay resident in HBM (their own buffers: a stateless lwse_sweep_ds_* call
+ * and the LWS resident tables / ticks never touch them).  Watch events arrive as row patches
+ * (lwse_patch_seg with LWSE_TABLE_DS / _DS_ROLES / _DS_REVROLES, consumed in place when they lie in
+ * the arena, staged otherwise; LWSE_PATCH_RANGE as for the LWS tick), one call returns the result rows
+ * that changed:   patches -> scatter kernel -> resident DS sweep -> publish kernel   (engine stream)
+ * and the host spins on a sequence word in pinned memory: no stream synchronize, no device->host
+ * copy-engine transfer on the path.  The results equal lwse_sweep_ds_* on the same tables.  Replaces,
+ * per reconcile pass, GetRevisionRolesList -> List (lws_manager.go:161-213) for every DS.
+ *
+ * Change lists.  A DS is VALID in a tick when the sweep does not flag it LWSE_DOUT_BAD_TABLE.  The
+ * rows a valid DS OWNS are role rows [role_base, role_base + n_roles) and revision-role rows
+ * [rev_base, rev_base + (n_old_revs + 1) * n_roles).  Every result row has a COMMITTED value: the last
+ * value a tick wrote to it (zero bytes if none did since lwse_ds_resident_load).
+ *   - a role / revision-role row is listed when a valid DS owns it and its new value differs from its
+ *     committed value, or this is the first tick after lwse_ds_resident_load;
+ *   - a DS row is listed when its ds_out differs from its committed value, or any of its role /
+ *     revision-role rows is listed, or this is the first tick after a load: the list is the set of DS
+ *     keys that need work, always with the current ds_out;
+ *   - a DS flagged BAD_TABLE writes only its ds_out; the rows it used to own keep their committed
+ *     values and are not listed.
+ * Invariant: a zero mirror with every tick's lists applied in order equals lwse_ds_resident_outputs
+ * on every row (and, on the rows valid DSes own, the stateless sweep of the same tables).
+ * Like every other resident call, a DS resident call first waits for (and drops the results of) the
+ * LWS ticks in flight.  One DS tick runs at a time. */
+typedef struct lwse_ds_tick {
+  /* in */
+  const lwse_patch_seg* segs; /* tables LWSE_TABLE_DS .. LWSE_TABLE_DS_REVROLES only */
+  uint32_t n_segs;            /* <= LWSE_TICK_MAX_SEGS */
+  uint32_t flags;             /* reserved, 0 */
+  /* out: views of engine-owned pinned memory, valid until the next lwse_*resident* call on this
+   * engine.  n_* counts the listed rows (at most the table's rows).  Order is unspecified. */
+  const uint32_t* ds_rows;
+  const lwse_ds_out* ds_out;
+  uint32_t n_ds;
+  uint32_t n_roles;
+  const uint32_t* role_rows;
+  const lwse_ds_role_out* role_out;
+  const uint32_t* revrole_rows;
+  const lwse_ds_revrole_out* revrole_out;
+  uint32_t n_revroles;
+  uint32_t reserved;
+} lwse_ds_tick;
+
+/* Copy the three input tables of `host` to the device, where they stay resident; output pointers are
+ * ignored.  Previous results are forgotten: committed outputs start at zero bytes. */
+LWSE_API int lwse_ds_resident_load(lwse_engine* e, const lwse_ds_tables* host);
+LWSE_API int lwse_ds_resident_tick(lwse_engine* e, lwse_ds_tick* t);
+/* Every committed result row (n_ds / n_roles / n_revroles rows of the loaded tables; NULL skips). */
+LWSE_API int lwse_ds_resident_outputs(lwse_engine* e, lwse_ds_out* ds_out, lwse_ds_role_out* role_out,
+                                      lwse_ds_revrole_out* revrole_out);
 
 /* ------------------------------------------------------------------------- */
 /* Group / subgroup keys (SHA-1) and subgroup indices                        */

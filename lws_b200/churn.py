@@ -166,3 +166,64 @@ class ArenaPlan:
         view[...] = a.reshape(-1) if a.dtype.fields is None else a
         self._cursor = off + a.nbytes
         return view
+
+
+# --------------------------------------------------------------------------- #
+# DisaggregatedSet tables (lwse_ds_resident_tick)
+# --------------------------------------------------------------------------- #
+@dataclass
+class DsPatchSet:
+    """One reconcile pass of the DS controller's work queue, as row patches (rows sorted, distinct)."""
+
+    rr_rows: np.ndarray
+    rr_vals: np.ndarray
+    role_rows: np.ndarray = field(default_factory=lambda: np.zeros(0, np.uint32))
+    role_vals: np.ndarray = field(default_factory=lambda: R.aligned_empty(0, R.DS_ROLE_REC))
+
+    def h2d_bytes(self) -> int:
+        return int(self.rr_rows.nbytes + self.rr_vals.nbytes + self.role_rows.nbytes + self.role_vals.nbytes)
+
+
+def make_ds_plan(t, sweep_ds, frac_revroles: float, n_sets: int = 4, frac_target: float = 0.001,
+                 seed: int = 11) -> list[DsPatchSet]:
+    """Patch sets for DS tables ``t`` (a ``synth.DsTables``), simulated once from its state:
+    in every set a fraction ``frac_revroles`` of the (revision, role) rows where an LWS exists
+    applies the previous sweep's decision (``replicas ← revrole_out``: the controller scaled the
+    child) and half of those become ready (``ready_replicas ← replicas``); about ``frac_target``
+    of the spec roles get a new ``target_replicas``.  ``sweep_ds(ds, roles, revroles)`` is the
+    sweep the decisions come from (the oracle).  The layout never changes: no row moves, no
+    child LWS appears or goes, so every set is valid for the resident tables of ``t``."""
+    rng = np.random.Generator(np.random.PCG64(seed))
+    roles, rr = t.roles.copy(), t.revroles.copy()
+    exists = np.flatnonzero((rr["flags"] & R.RR_EXISTS) != 0)
+    in_spec = np.flatnonzero((roles["flags"] & R.ROLE_IN_SPEC) != 0)
+    n_rr = int(round(len(exists) * frac_revroles))
+    n_ro = int(round(len(in_spec) * frac_target))
+    sets = []
+    for _ in range(n_sets):
+        _, _, rr_out = sweep_ds(t.ds, roles, rr)
+        rows = np.sort(rng.choice(exists, size=min(n_rr, len(exists)), replace=False)).astype(np.uint32)
+        want = rr_out[rows]
+        scaled = want >= 0
+        rr["replicas"][rows[scaled]] = want[scaled]
+        rr["flags"][rows[scaled]] &= np.uint32(~R.RR_REPLICAS_NIL & 0xFFFFFFFF)
+        ready = rows[rng.random(len(rows)) < 0.5]
+        rr["ready_replicas"][ready] = rr["replicas"][ready]
+        rv = R.aligned_empty(len(rows), R.DS_REVROLE_REC)
+        rv[:] = rr[rows]
+        ps = DsPatchSet(rows, rv)
+        if n_ro:
+            ro = np.sort(rng.choice(in_spec, size=min(n_ro, len(in_spec)), replace=False)).astype(np.uint32)
+            roles["target_replicas"][ro] = np.maximum(roles["target_replicas"][ro] + rng.choice(np.array([-1, 1]), len(ro)), 0)
+            vals = R.aligned_empty(len(ro), R.DS_ROLE_REC)
+            vals[:] = roles[ro]
+            ps.role_rows, ps.role_vals = ro, vals
+        sets.append(ps)
+    return sets
+
+
+def apply_ds_to_mirror(ps: DsPatchSet, roles: np.ndarray, revroles: np.ndarray) -> None:
+    """The host-side mirror of one DS tick's patches."""
+    revroles[ps.rr_rows] = ps.rr_vals
+    if len(ps.role_rows):
+        roles[ps.role_rows] = ps.role_vals

@@ -161,23 +161,28 @@ __device__ bool compute_next_step(int n, const int* initial_old, const int* cur_
   return false;
 }
 
-__global__ void __launch_bounds__(128) ds_sweep_kernel(const lwse_ds_tables t) {
-  for (uint32_t d = blockIdx.x * blockDim.x + threadIdx.x; d < t.n_ds; d += gridDim.x * blockDim.x) {
-    const uint4 h0 = ldg_stream(reinterpret_cast<const uint4*>(t.ds + d) + 0);
-    const uint4 h1 = ldg_stream(reinterpret_cast<const uint4*>(t.ds + d) + 1);
+// A DS record's row ranges lie inside the tables (else the DS is flagged LWSE_DOUT_BAD_TABLE).
+__device__ __forceinline__ bool ds_in_tables(const lwse_ds_tables& t, const uint4 h0, const uint4 h1) {
+  const uint32_t role_base = h0.z, n_roles = h0.w, n_spec = h1.x, rev_base = h1.y, n_old = h1.z;
+  return !(n_roles > LWSE_DS_MAX_ROLES || n_spec > n_roles || n_old > LWSE_DS_MAX_OLD_REVS ||
+           (uint64_t)role_base + n_roles > t.n_roles ||
+           (uint64_t)rev_base + (uint64_t)(n_old + 1u) * n_roles > t.n_revroles);
+}
+
+// The decisions of one DS (record words h0, h1; its ranges checked by ds_in_tables): the role rows go
+// to role_out, the (revision, role) rows to revrole_out — both indexed like the input tables.
+// revrole_out is working storage as well: scaleDownOld reads back what scaleUpNew / reconcileSimple
+// wrote.  Returns the ds_out row.
+__device__ __forceinline__ uint4 ds_decide(const lwse_ds_tables& t, const uint4 h0, const uint4 h1,
+                                           lwse_ds_role_out* role_out, lwse_ds_revrole_out* revrole_out) {
+  {
     const uint32_t role_base = h0.z, n_roles = h0.w, n_spec = h1.x, rev_base = h1.y, n_old = h1.z, dflags = h1.w;
     uint32_t oflags = 0, drained = 0, ready_revs = 0;
     const int n = (int)n_roles, S = (int)n_spec, V = (int)n_old;
-    if (n_roles > LWSE_DS_MAX_ROLES || n_spec > n_roles || n_old > LWSE_DS_MAX_OLD_REVS ||
-        (uint64_t)role_base + n_roles > t.n_roles ||
-        (uint64_t)rev_base + (uint64_t)(n_old + 1u) * n_roles > t.n_revroles) {
-      stg_stream(t.ds_out + d, make_uint4(LWSE_DOUT_BAD_TABLE, 0, 0, 0));
-      continue;
-    }
     const lwse_ds_role_rec* roles = t.roles + role_base;
     const uint4* rr = reinterpret_cast<const uint4*>(t.revroles + rev_base);  // {replicas, initial, ready, flags}
-    lwse_ds_role_out* ro = t.role_out + role_base;
-    lwse_ds_revrole_out* rro = t.revrole_out + rev_base;
+    lwse_ds_role_out* ro = role_out + role_base;
+    lwse_ds_revrole_out* rro = revrole_out + rev_base;
 
     int initial_old[MAXR], cur_old[MAXR], cur_new[MAXR], target[MAXR];
     RuConfig cfg[MAXR];
@@ -310,7 +315,127 @@ __global__ void __launch_bounds__(128) ds_sweep_kernel(const lwse_ds_tables t) {
         }
       }
     }
-    stg_stream(t.ds_out + d, make_uint4(oflags, drained, ready_revs, 0));
+    return make_uint4(oflags, drained, ready_revs, 0);
+  }
+}
+
+// Resident form (lwse_ds_resident_tick): the tables are the engine's resident ones; the decisions go
+// to scratch rows, and every row a valid DS owns is compared with its committed value — rows that
+// differ (all rows on the first tick after a load) are written back and appended to the change lists.
+struct DsResidentArgs {
+  lwse_ds_out* ds_committed;
+  lwse_ds_role_out* role_committed;
+  lwse_ds_revrole_out* revrole_committed;
+  lwse_ds_role_out* role_scratch;
+  lwse_ds_revrole_out* revrole_scratch;
+  uint32_t* ds_rows;  // change lists (device memory), capacity = table rows
+  lwse_ds_out* ds_outs;
+  uint32_t* role_rows;
+  lwse_ds_role_out* role_outs;
+  uint32_t* revrole_rows;
+  lwse_ds_revrole_out* revrole_outs;
+  uint32_t* counts;  // [0] ds, [1] role, [2] revrole rows listed
+  uint32_t first;    // first tick after a load: list every row
+};
+
+// Warp-aggregated append: every lane of the warp calls this; lane i reserves n_i slots of *counter with
+// one atomic for the whole warp.  Returns lane i's first slot.
+__device__ __forceinline__ uint32_t warp_reserve(uint32_t* counter, uint32_t n) {
+  const uint32_t lane = threadIdx.x & 31u;
+  uint32_t incl = n;
+#pragma unroll
+  for (uint32_t o = 1; o < 32u; o <<= 1) {
+    const uint32_t v = __shfl_up_sync(0xFFFFFFFFu, incl, o);
+    if (lane >= o) incl += v;
+  }
+  const uint32_t total = __shfl_sync(0xFFFFFFFFu, incl, 31);
+  uint32_t base = 0;
+  if (total) {
+    if (lane == 31u) base = atomicAdd(counter, total);
+    base = __shfl_sync(0xFFFFFFFFu, base, 31);
+  }
+  return base + incl - n;
+}
+
+__device__ __forceinline__ bool ne(const lwse_ds_role_out a, const lwse_ds_role_out b) {
+  return a.next_old != b.next_old || a.next_new != b.next_new;
+}
+__device__ __forceinline__ bool ne(const uint4 a, const uint4 b) { return a.x != b.x || a.y != b.y || a.z != b.z || a.w != b.w; }
+
+template <bool kResident>
+__global__ void __launch_bounds__(128) ds_sweep_kernel(const lwse_ds_tables t, const DsResidentArgs r) {
+  if constexpr (!kResident) {
+    for (uint32_t d = blockIdx.x * blockDim.x + threadIdx.x; d < t.n_ds; d += gridDim.x * blockDim.x) {
+      const uint4 h0 = ldg_stream(reinterpret_cast<const uint4*>(t.ds + d) + 0);
+      const uint4 h1 = ldg_stream(reinterpret_cast<const uint4*>(t.ds + d) + 1);
+      if (!ds_in_tables(t, h0, h1)) {
+        stg_stream(t.ds_out + d, make_uint4(LWSE_DOUT_BAD_TABLE, 0, 0, 0));
+        continue;
+      }
+      stg_stream(t.ds_out + d, ds_decide(t, h0, h1, t.role_out, t.revrole_out));
+    }
+  } else {
+    pdl_launch_dependents();
+    pdl_wait_prior();  // the kernel before this one (the tick's patch scatter) writes the input tables
+    // whole warps iterate together: the list appends are warp-collective
+    const uint32_t n_iter = (t.n_ds + 31u) & ~31u;
+    for (uint32_t d = blockIdx.x * blockDim.x + threadIdx.x; d < n_iter; d += gridDim.x * blockDim.x) {
+      const bool live = d < t.n_ds;
+      uint4 h0 = make_uint4(0, 0, 0, 0), h1 = h0, o = h0;
+      bool valid = false;
+      if (live) {
+        h0 = ldg_stream(reinterpret_cast<const uint4*>(t.ds + d) + 0);
+        h1 = ldg_stream(reinterpret_cast<const uint4*>(t.ds + d) + 1);
+        valid = ds_in_tables(t, h0, h1);
+        o = valid ? ds_decide(t, h0, h1, r.role_scratch, r.revrole_scratch) : make_uint4(LWSE_DOUT_BAD_TABLE, 0, 0, 0);
+      }
+      const uint32_t role_base = h0.z, n = valid ? h0.w : 0u, rev_base = h1.y;
+      const uint32_t n_rr = valid ? (h1.z + 1u) * n : 0u;
+      const bool first = r.first != 0u;
+      // pass 1: how many rows of each list this DS appends
+      uint32_t c_role = 0, c_rr = 0;
+      for (uint32_t i = 0; i < n; i++)
+        c_role += (first || ne(r.role_scratch[role_base + i], r.role_committed[role_base + i])) ? 1u : 0u;
+      for (uint32_t k = 0; k < n_rr; k++)
+        c_rr += (first || r.revrole_scratch[rev_base + k] != r.revrole_committed[rev_base + k]) ? 1u : 0u;
+      const uint4 committed = live ? *reinterpret_cast<const uint4*>(r.ds_committed + d) : o;
+      const uint32_t c_ds = live && (first || ne(o, committed) || c_role || c_rr) ? 1u : 0u;
+      uint32_t at_role = warp_reserve(r.counts + 1, c_role);
+      uint32_t at_rr = warp_reserve(r.counts + 2, c_rr);
+      const uint32_t at_ds = warp_reserve(r.counts + 0, c_ds);
+      // pass 2: write back and list the rows that changed
+      if (c_role)
+        for (uint32_t i = 0; i < n; i++) {
+          const uint32_t row = role_base + i;
+          const lwse_ds_role_out v = r.role_scratch[row];
+          if (!first && !ne(v, r.role_committed[row])) continue;
+          r.role_committed[row] = v;
+          if (at_role < t.n_roles) {
+            r.role_rows[at_role] = row;
+            r.role_outs[at_role] = v;
+          }
+          at_role++;
+        }
+      if (c_rr)
+        for (uint32_t k = 0; k < n_rr; k++) {
+          const uint32_t row = rev_base + k;
+          const lwse_ds_revrole_out v = r.revrole_scratch[row];
+          if (!first && v == r.revrole_committed[row]) continue;
+          r.revrole_committed[row] = v;
+          if (at_rr < t.n_revroles) {
+            r.revrole_rows[at_rr] = row;
+            r.revrole_outs[at_rr] = v;
+          }
+          at_rr++;
+        }
+      if (c_ds) {
+        *reinterpret_cast<uint4*>(r.ds_committed + d) = o;
+        if (at_ds < t.n_ds) {
+          r.ds_rows[at_ds] = d;
+          *reinterpret_cast<uint4*>(r.ds_outs + at_ds) = o;
+        }
+      }
+    }
   }
 }
 
@@ -319,8 +444,24 @@ int launch_ds_sweep(const lwse_ds_tables* t, int sm_count, cudaStream_t s, int* 
   if (t->n_ds == 0) return 0;
   const uint32_t want = (t->n_ds + 127u) / 128u;
   const uint32_t cap = (uint32_t)sm_count * 16u;
-  ds_sweep_kernel<<<want < cap ? want : cap, 128, 0, s>>>(*t);
+  ds_sweep_kernel<false><<<want < cap ? want : cap, 128, 0, s>>>(*t, DsResidentArgs{});
   cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) {
+    *cuda_err = (int)e;
+    return -1;
+  }
+  return 1;
+}
+
+// pdl: launched programmatically dependent on the kernel before it (which may write the input tables:
+// the resident kernel waits at its top either way).
+int launch_ds_resident_sweep(const lwse_ds_tables* t, const DsResidentArgs* r, int sm_count, cudaStream_t s, bool pdl,
+                             int* cuda_err) {
+  *cuda_err = 0;
+  if (t->n_ds == 0) return 0;
+  const uint32_t want = (t->n_ds + 127u) / 128u;
+  const uint32_t cap = (uint32_t)sm_count * 16u;
+  const cudaError_t e = launch_pdl(ds_sweep_kernel<true>, dim3(want < cap ? want : cap), dim3(128), 0, s, pdl, *t, *r);
   if (e != cudaSuccess) {
     *cuda_err = (int)e;
     return -1;

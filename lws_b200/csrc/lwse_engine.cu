@@ -98,6 +98,23 @@ int launch_place_diff(const lwse_place_out* d_cur, lwse_place_out* d_prev, uint3
                       lwse_place_out* d_outs, uint32_t capacity, uint32_t* d_count, cudaStream_t s, int* cuda_err);
 // lwse_ds_kernels.cu
 int launch_ds_sweep(const lwse_ds_tables* t, int sm_count, cudaStream_t s, int* cuda_err);
+struct DsResidentArgs {
+  lwse_ds_out* ds_committed;
+  lwse_ds_role_out* role_committed;
+  lwse_ds_revrole_out* revrole_committed;
+  lwse_ds_role_out* role_scratch;
+  lwse_ds_revrole_out* revrole_scratch;
+  uint32_t* ds_rows;
+  lwse_ds_out* ds_outs;
+  uint32_t* role_rows;
+  lwse_ds_role_out* role_outs;
+  uint32_t* revrole_rows;
+  lwse_ds_revrole_out* revrole_outs;
+  uint32_t* counts;
+  uint32_t first;
+};
+int launch_ds_resident_sweep(const lwse_ds_tables* t, const DsResidentArgs* r, int sm_count, cudaStream_t s, bool pdl,
+                             int* cuda_err);
 // lwse_sha1_kernels.cu
 int launch_sha1(const uint8_t* d_bytes, const uint32_t* d_offsets, uint32_t n, uint8_t* d_digests,
                 int sm_count, cudaStream_t s, int* cuda_err);
@@ -261,6 +278,17 @@ struct lwse_engine {
   const uint32_t* place_counters = nullptr;  // device: counters / phase stamps of the last placement call
   const uint32_t* place_unpinned = nullptr;  // device: its unpinned-request count
   DevBuf ds, ds_roles, ds_revroles, ds_out, ds_role_out, ds_revrole_out;
+  // resident DS tables (lwse_ds_resident_*): inputs, committed outputs, scratch, change lists — none
+  // shared with the stateless DS sweep's staging above or with the LWS resident state
+  DevBuf rd_ds, rd_roles, rd_revroles, rd_ds_out, rd_role_out, rd_revrole_out, rd_role_scratch, rd_revrole_scratch;
+  DevBuf rd_chg_dev;                 // change lists: [ds rows | ds out | role rows | role out | revrole rows | revrole out]
+  DevBuf rd_counts;                  // [0] ds [1] role [2] revrole rows listed, [3] publish ticket
+  PinBuf rd_chg;                     // the same layout in pinned, mapped memory (the publish kernel copies into it)
+  PinBuf rd_tickw;                   // [0..2] the three counts, [4] sequence word
+  size_t rd_chg_off[6] = {};
+  uint32_t rdn_ds = 0, rdn_roles = 0, rdn_revroles = 0;
+  uint32_t rd_seq = 0, rd_last_changed = 0;
+  bool rd_loaded = false, rd_first = false;
   DevBuf sha_bytes, sha_offsets, sha_digests, sha_ints;
   uint32_t* h_rounds = nullptr;  // pinned
   // peer exchange of the multi-GPU placement step (lwse_exchange_*)
@@ -472,9 +500,11 @@ LWSE_API void lwse_destroy(lwse_engine* e) {
                       &e->ds_role_out, &e->ds_revrole_out, &e->sha_bytes, &e->sha_offsets, &e->sha_digests, &e->sha_ints,
                       &e->r_lws, &e->r_groups, &e->r_pst, &e->r_pid, &e->r_lws_out, &e->r_group_out, &e->r_scan,
                       &e->r_counts, &e->r_occ, &e->r_preq, &e->r_pout, &e->r_pout_prev, &e->h_counts_dev, &e->place_ns_scratch,
-                      &e->arena_mirror, &e->stage_mirror, &e->chg_dev, &e->tdesc_dev};
+                      &e->arena_mirror, &e->stage_mirror, &e->chg_dev, &e->tdesc_dev,
+                      &e->rd_ds, &e->rd_roles, &e->rd_revroles, &e->rd_ds_out, &e->rd_role_out, &e->rd_revrole_out,
+                      &e->rd_role_scratch, &e->rd_revrole_scratch, &e->rd_chg_dev, &e->rd_counts};
     for (DevBuf* b : bufs) b->release();
-    PinBuf* pins[] = {&e->arena, &e->stage, &e->chg, &e->tickw, &e->tdesc};
+    PinBuf* pins[] = {&e->arena, &e->stage, &e->chg, &e->tickw, &e->tdesc, &e->rd_chg, &e->rd_tickw};
     for (PinBuf* b : pins) b->release();
     if (e->ev_place) cudaEventDestroy(e->ev_place);
     if (e->h_rounds) cudaFreeHost(e->h_rounds);
@@ -780,8 +810,18 @@ LWSE_API int lwse_resident_arena(lwse_engine* e, uint64_t min_bytes, void** base
   return LWSE_OK;
 }
 
-// table → (device base, rows, bytes per row)
-static bool resident_table(lwse_engine* e, uint32_t which, void** base, uint64_t* rows, uint32_t* row_bytes) {
+// table → (device base, rows, bytes per row).  `ds`: the tables of the DS tick (ids 5-7), which the
+// LWS tick does not take; the DS tick takes nothing else.
+static bool resident_table(lwse_engine* e, uint32_t which, void** base, uint64_t* rows, uint32_t* row_bytes, bool ds = false) {
+  if (ds) {
+    switch (which) {
+      case LWSE_TABLE_DS: *base = e->rd_ds.p; *rows = e->rdn_ds; *row_bytes = sizeof(lwse_ds_rec); return true;
+      case LWSE_TABLE_DS_ROLES: *base = e->rd_roles.p; *rows = e->rdn_roles; *row_bytes = sizeof(lwse_ds_role_rec); return true;
+      case LWSE_TABLE_DS_REVROLES:
+        *base = e->rd_revroles.p; *rows = e->rdn_revroles; *row_bytes = sizeof(lwse_ds_revrole_rec); return true;
+      default: return false;
+    }
+  }
   switch (which) {
     case LWSE_TABLE_LWS: *base = e->r_lws.p; *rows = e->rn_lws; *row_bytes = sizeof(lwse_lws_rec); return true;
     case LWSE_TABLE_GROUPS: *base = e->r_groups.p; *rows = e->rn_groups; *row_bytes = sizeof(lwse_group_rec); return true;
@@ -839,7 +879,7 @@ static int launch_scatter_plan(lwse_engine* e, const ScatterPlan& p, cudaStream_
 static int apply_patches_locked(lwse_engine* e, const lwse_patch_seg* segs, uint32_t n_segs, bool* wrote,
                                 uint32_t tables = 0xFFFFFFFFu, cudaStream_t s = nullptr, size_t stage_base = 0,
                                 size_t* stage_used = nullptr, long dma_min_bytes = 0, ScatterPlan* defer = nullptr,
-                                bool plan_only = false) {
+                                bool plan_only = false, bool ds = false) {
   *wrote = false;
   if (stage_used) *stage_used = stage_base;
   if (n_segs == 0) return LWSE_OK;
@@ -851,7 +891,7 @@ static int apply_patches_locked(lwse_engine* e, const lwse_patch_seg* segs, uint
     void* base;
     uint64_t rows;
     uint32_t rb;
-    if (!resident_table(e, segs[i].table, &base, &rows, &rb)) return LWSE_ERR_INVALID_ARG;
+    if (!resident_table(e, segs[i].table, &base, &rows, &rb, ds)) return LWSE_ERR_INVALID_ARG;
     if (segs[i].n == 0 || !((tables >> segs[i].table) & 1u)) continue;
     if (!segs[i].values || (!(segs[i].flags & LWSE_PATCH_RANGE) && !segs[i].rows)) return LWSE_ERR_INVALID_ARG;
     if (segs[i].flags & LWSE_PATCH_RANGE) {
@@ -878,7 +918,7 @@ static int apply_patches_locked(lwse_engine* e, const lwse_patch_seg* segs, uint
     void* base;
     uint64_t rows;
     uint32_t rb;
-    resident_table(e, g.table, &base, &rows, &rb);
+    resident_table(e, g.table, &base, &rows, &rb, ds);
     *wrote = true;
     if (g.table == LWSE_TABLE_PLACE_REQS && e->r_place_grouped) {
       // a request that moves to another namespace breaks the grouping the fast placement kernels rely on
@@ -2114,6 +2154,155 @@ LWSE_API int lwse_sweep_ds_host(lwse_engine* e, const lwse_ds_tables* h) {
   if (o_ds) LWSE_CUDA(e, cudaMemcpyAsync(h->ds_out, e->ds_out.p, o_ds, cudaMemcpyDeviceToHost, s));
   if (o_ro) LWSE_CUDA(e, cudaMemcpyAsync(h->role_out, e->ds_role_out.p, o_ro, cudaMemcpyDeviceToHost, s));
   if (o_rr) LWSE_CUDA(e, cudaMemcpyAsync(h->revrole_out, e->ds_revrole_out.p, o_rr, cudaMemcpyDeviceToHost, s));
+  LWSE_CUDA(e, cudaStreamSynchronize(s));
+  return LWSE_OK;
+}
+
+// ---------------------------------------------------------------------------
+// Resident DisaggregatedSet tables
+// ---------------------------------------------------------------------------
+LWSE_API int lwse_ds_resident_load(lwse_engine* e, const lwse_ds_tables* h) {
+  if (!e || !h) return LWSE_ERR_INVALID_ARG;
+  if ((h->n_ds && !h->ds) || (h->n_roles && !h->roles) || (h->n_revroles && !h->revroles)) return LWSE_ERR_INVALID_ARG;
+  std::lock_guard<std::mutex> lock(e->mu);
+  DeviceGuard guard(e->device);
+  {
+    const int drc = drain_ticks_locked(e);
+    if (drc != LWSE_OK) return drc;
+  }
+  cudaStream_t s = e->stream;
+  LWSE_CUDA(e, cudaStreamSynchronize(s));  // (the previous DS tick's publish kernel is done with the lists)
+  e->rd_loaded = false;
+  const size_t b_ds = (size_t)h->n_ds * sizeof(lwse_ds_rec), b_ro = (size_t)h->n_roles * sizeof(lwse_ds_role_rec),
+               b_rr = (size_t)h->n_revroles * sizeof(lwse_ds_revrole_rec);
+  const size_t o_ds = (size_t)h->n_ds * sizeof(lwse_ds_out), o_ro = (size_t)h->n_roles * sizeof(lwse_ds_role_out),
+               o_rr = (size_t)h->n_revroles * sizeof(lwse_ds_revrole_out);
+  LWSE_CUDA(e, e->rd_ds.reserve(b_ds + 16));
+  LWSE_CUDA(e, e->rd_roles.reserve(b_ro + 16));
+  LWSE_CUDA(e, e->rd_revroles.reserve(b_rr + 16));
+  LWSE_CUDA(e, e->rd_ds_out.reserve(o_ds + 16));
+  LWSE_CUDA(e, e->rd_role_out.reserve(o_ro + 16));
+  LWSE_CUDA(e, e->rd_revrole_out.reserve(o_rr + 16));
+  LWSE_CUDA(e, e->rd_role_scratch.reserve(o_ro + 16));
+  LWSE_CUDA(e, e->rd_revrole_scratch.reserve(o_rr + 16));
+  size_t off = 0;
+  const size_t sizes[6] = {(size_t)h->n_ds * 4, o_ds, (size_t)h->n_roles * 4, o_ro, (size_t)h->n_revroles * 4, o_rr};
+  for (int k = 0; k < 6; k++) {
+    e->rd_chg_off[k] = off;
+    off += align256(sizes[k] + 16);
+  }
+  LWSE_CUDA(e, e->rd_chg_dev.reserve(off));
+  LWSE_CUDA(e, e->rd_chg.reserve(off));
+  LWSE_CUDA(e, e->rd_counts.reserve(64));
+  LWSE_CUDA(e, e->rd_tickw.reserve(64));
+  LWSE_CUDA(e, cudaMemsetAsync(e->rd_counts.p, 0, 64, s));
+  if (b_ds) LWSE_CUDA(e, cudaMemcpyAsync(e->rd_ds.p, h->ds, b_ds, cudaMemcpyHostToDevice, s));
+  if (b_ro) LWSE_CUDA(e, cudaMemcpyAsync(e->rd_roles.p, h->roles, b_ro, cudaMemcpyHostToDevice, s));
+  if (b_rr) LWSE_CUDA(e, cudaMemcpyAsync(e->rd_revroles.p, h->revroles, b_rr, cudaMemcpyHostToDevice, s));
+  if (o_ds) LWSE_CUDA(e, cudaMemsetAsync(e->rd_ds_out.p, 0, o_ds, s));  // committed values start at zero bytes
+  if (o_ro) LWSE_CUDA(e, cudaMemsetAsync(e->rd_role_out.p, 0, o_ro, s));
+  if (o_rr) LWSE_CUDA(e, cudaMemsetAsync(e->rd_revrole_out.p, 0, o_rr, s));
+  LWSE_CUDA(e, cudaStreamSynchronize(s));
+  e->rdn_ds = h->n_ds;
+  e->rdn_roles = h->n_roles;
+  e->rdn_revroles = h->n_revroles;
+  e->rd_last_changed = 0;
+  e->rd_first = true;
+  e->rd_loaded = true;
+  return LWSE_OK;
+}
+
+LWSE_API int lwse_ds_resident_tick(lwse_engine* e, lwse_ds_tick* t) {
+  if (!e || !t || (t->n_segs && !t->segs) || t->n_segs > LWSE_TICK_MAX_SEGS || t->flags != 0) return LWSE_ERR_INVALID_ARG;
+  std::lock_guard<std::mutex> lock(e->mu);
+  if (!e->rd_loaded) return LWSE_ERR_NOT_READY;
+  DeviceGuard guard(e->device);
+  int rc = drain_ticks_locked(e);
+  if (rc != LWSE_OK) return rc;
+  cudaStream_t s = e->stream;
+  bool wrote = false;
+  rc = apply_patches_locked(e, t->segs, t->n_segs, &wrote, 0xFFFFFFFFu, s, 0, nullptr, 0, nullptr, false, /*ds=*/true);
+  if (rc != LWSE_OK) return rc;
+  uint8_t* chg_v = static_cast<uint8_t*>(e->rd_chg_dev.p);
+  uint8_t* chg_d = static_cast<uint8_t*>(e->rd_chg.d);
+  uint32_t* cnt = static_cast<uint32_t*>(e->rd_counts.p);
+  lwse_ds_tables d{};
+  d.ds = (const lwse_ds_rec*)e->rd_ds.p;
+  d.n_ds = e->rdn_ds;
+  d.roles = (const lwse_ds_role_rec*)e->rd_roles.p;
+  d.n_roles = e->rdn_roles;
+  d.revroles = (const lwse_ds_revrole_rec*)e->rd_revroles.p;
+  d.n_revroles = e->rdn_revroles;
+  lwse::DsResidentArgs r{};
+  r.ds_committed = (lwse_ds_out*)e->rd_ds_out.p;
+  r.role_committed = (lwse_ds_role_out*)e->rd_role_out.p;
+  r.revrole_committed = (lwse_ds_revrole_out*)e->rd_revrole_out.p;
+  r.role_scratch = (lwse_ds_role_out*)e->rd_role_scratch.p;
+  r.revrole_scratch = (lwse_ds_revrole_out*)e->rd_revrole_scratch.p;
+  r.ds_rows = reinterpret_cast<uint32_t*>(chg_v + e->rd_chg_off[0]);
+  r.ds_outs = reinterpret_cast<lwse_ds_out*>(chg_v + e->rd_chg_off[1]);
+  r.role_rows = reinterpret_cast<uint32_t*>(chg_v + e->rd_chg_off[2]);
+  r.role_outs = reinterpret_cast<lwse_ds_role_out*>(chg_v + e->rd_chg_off[3]);
+  r.revrole_rows = reinterpret_cast<uint32_t*>(chg_v + e->rd_chg_off[4]);
+  r.revrole_outs = reinterpret_cast<lwse_ds_revrole_out*>(chg_v + e->rd_chg_off[5]);
+  r.counts = cnt;
+  r.first = e->rd_first ? 1u : 0u;
+  int cuda_err = 0;
+  // behind the scatter kernel: programmatically dependent, the sweep waits at its top
+  int launched = lwse::launch_ds_resident_sweep(&d, &r, e->sm_count, s, wrote, &cuda_err);
+  if (launched < 0) return fail_cuda(e, (cudaError_t)cuda_err);
+  e->launches += (uint64_t)launched;
+  lwse::PublishListHost pl[3] = {
+      {r.ds_rows, r.ds_outs, reinterpret_cast<uint32_t*>(chg_d + e->rd_chg_off[0]), chg_d + e->rd_chg_off[1], cnt + 0, e->rdn_ds,
+       (uint32_t)sizeof(lwse_ds_out)},
+      {r.role_rows, r.role_outs, reinterpret_cast<uint32_t*>(chg_d + e->rd_chg_off[2]), chg_d + e->rd_chg_off[3], cnt + 1,
+       e->rdn_roles, (uint32_t)sizeof(lwse_ds_role_out)},
+      {r.revrole_rows, r.revrole_outs, reinterpret_cast<uint32_t*>(chg_d + e->rd_chg_off[4]), chg_d + e->rd_chg_off[5], cnt + 2,
+       e->rdn_revroles, (uint32_t)sizeof(lwse_ds_revrole_out)}};
+  uint32_t seq = ++e->rd_seq;
+  if (seq == 0) seq = ++e->rd_seq;
+  launched = lwse::launch_publish(pl, nullptr, static_cast<uint32_t*>(e->rd_tickw.d), 4, seq, cnt + 3, e->rd_last_changed, s,
+                                  &cuda_err, nullptr, 0, /*pdl=*/launched > 0);
+  if (launched < 0) return fail_cuda(e, (cudaError_t)cuda_err);
+  e->launches += (uint64_t)launched;
+  volatile uint32_t* hw = static_cast<volatile uint32_t*>(e->rd_tickw.h);
+  cudaError_t werr = cudaSuccess;
+  if (!wait_word(hw + 4, seq, s, &werr)) {
+    const cudaError_t a = cudaStreamSynchronize(s);
+    return fail_cuda(e, werr != cudaSuccess ? werr : a != cudaSuccess ? a : cudaErrorUnknown);
+  }
+  const uint8_t* base = static_cast<const uint8_t*>(e->rd_chg.h);
+  t->n_ds = hw[0] < e->rdn_ds ? hw[0] : e->rdn_ds;
+  t->n_roles = hw[1] < e->rdn_roles ? hw[1] : e->rdn_roles;
+  t->n_revroles = hw[2] < e->rdn_revroles ? hw[2] : e->rdn_revroles;
+  t->ds_rows = reinterpret_cast<const uint32_t*>(base + e->rd_chg_off[0]);
+  t->ds_out = reinterpret_cast<const lwse_ds_out*>(base + e->rd_chg_off[1]);
+  t->role_rows = reinterpret_cast<const uint32_t*>(base + e->rd_chg_off[2]);
+  t->role_out = reinterpret_cast<const lwse_ds_role_out*>(base + e->rd_chg_off[3]);
+  t->revrole_rows = reinterpret_cast<const uint32_t*>(base + e->rd_chg_off[4]);
+  t->revrole_out = reinterpret_cast<const lwse_ds_revrole_out*>(base + e->rd_chg_off[5]);
+  e->rd_last_changed = t->n_ds + t->n_roles + t->n_revroles;
+  e->rd_first = false;
+  return LWSE_OK;
+}
+
+LWSE_API int lwse_ds_resident_outputs(lwse_engine* e, lwse_ds_out* ds_out, lwse_ds_role_out* role_out,
+                                      lwse_ds_revrole_out* revrole_out) {
+  if (!e) return LWSE_ERR_INVALID_ARG;
+  std::lock_guard<std::mutex> lock(e->mu);
+  if (!e->rd_loaded) return LWSE_ERR_NOT_READY;
+  DeviceGuard guard(e->device);
+  int rc = drain_ticks_locked(e);
+  if (rc != LWSE_OK) return rc;
+  cudaStream_t s = e->stream;
+  if (ds_out && e->rdn_ds)
+    LWSE_CUDA(e, cudaMemcpyAsync(ds_out, e->rd_ds_out.p, (size_t)e->rdn_ds * sizeof(lwse_ds_out), cudaMemcpyDeviceToHost, s));
+  if (role_out && e->rdn_roles)
+    LWSE_CUDA(e, cudaMemcpyAsync(role_out, e->rd_role_out.p, (size_t)e->rdn_roles * sizeof(lwse_ds_role_out),
+                                 cudaMemcpyDeviceToHost, s));
+  if (revrole_out && e->rdn_revroles)
+    LWSE_CUDA(e, cudaMemcpyAsync(revrole_out, e->rd_revrole_out.p, (size_t)e->rdn_revroles * sizeof(lwse_ds_revrole_out),
+                                 cudaMemcpyDeviceToHost, s));
   LWSE_CUDA(e, cudaStreamSynchronize(s));
   return LWSE_OK;
 }

@@ -1151,7 +1151,8 @@ struct PublishList {
   uint4* dst_outs;      // mapped host
   uint32_t* count;      // device counter (reset here); null = list not in this tick
   uint32_t capacity;
-  uint32_t out_vec;     // uint4 per result row
+  uint32_t out_vec;     // uint4 per result row (rows of 16-byte multiples), else 0
+  uint32_t out_words;   // 32-bit words per result row of rows narrower than 16 bytes, else 0
 };
 struct PublishArgs {
   PublishList list[3];
@@ -1195,6 +1196,8 @@ __global__ void __launch_bounds__(kPublishThreads) publish_lists_kernel(const Pu
     for (uint32_t i = gtid + gsize; i < n; i += gsize) l.dst_rows[i] = __ldcg(l.src_rows + i);
 #pragma unroll 4
     for (uint32_t i = gtid + gsize; i < n * l.out_vec; i += gsize) l.dst_outs[i] = __ldcg(l.src_outs + i);
+    for (uint32_t i = gtid; i < n * l.out_words; i += gsize)  // (DS role / revision-role rows: 8 and 4 bytes)
+      reinterpret_cast<uint32_t*>(l.dst_outs)[i] = __ldcg(reinterpret_cast<const uint32_t*>(l.src_outs) + i);
   }
   __syncthreads();
   bool last = true;
@@ -1242,9 +1245,12 @@ int launch_publish(const PublishListHost* lists, const uint32_t* d_extra, uint32
                    uint32_t* d_clear, uint32_t n_clear, bool pdl) {
   *cuda_err = 0;
   PublishArgs a{};
-  for (int k = 0; k < 3; k++)
+  for (int k = 0; k < 3; k++) {
+    const bool vec = lists[k].out_bytes % 16u == 0;
     a.list[k] = PublishList{lists[k].src_rows, static_cast<const uint4*>(lists[k].src_outs), lists[k].dst_rows,
-                            static_cast<uint4*>(lists[k].dst_outs), lists[k].count, lists[k].capacity, lists[k].out_bytes / 16u};
+                            static_cast<uint4*>(lists[k].dst_outs), lists[k].count, lists[k].capacity,
+                            vec ? lists[k].out_bytes / 16u : 0u, vec ? 0u : lists[k].out_bytes / 4u};
+  }
   a.extra = d_extra;
   a.host_words = h_words;
   a.seq_slot = seq_slot;

@@ -81,6 +81,9 @@ SYMBOLS = {
     "lwse_exchange_status": ([C.c_void_p, C.POINTER(C.c_uint32)], C.c_int),
     "lwse_sweep_ds_host": ([C.c_void_p, C.POINTER(R.DsTables)], C.c_int),
     "lwse_sweep_ds_device": ([C.c_void_p, C.POINTER(R.DsTables), C.c_void_p], C.c_int),
+    "lwse_ds_resident_load": ([C.c_void_p, C.POINTER(R.DsTables)], C.c_int),
+    "lwse_ds_resident_tick": ([C.c_void_p, C.POINTER(R.DsTick)], C.c_int),
+    "lwse_ds_resident_outputs": ([C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p], C.c_int),
     "lwse_group_keys_host": ([C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p], C.c_int),
     "lwse_subgroup_keys_host": (
         [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p], C.c_int),
@@ -279,7 +282,8 @@ class Engine:
         self._chg = None
 
     _DT = {R.TABLE_LWS: R.LWS_REC, R.TABLE_GROUPS: R.GROUP_REC, R.TABLE_POD_STATE: R.POD_STATE,
-           R.TABLE_POD_IDENT: R.POD_IDENT, R.TABLE_PLACE_REQS: R.PLACE_REQ}
+           R.TABLE_POD_IDENT: R.POD_IDENT, R.TABLE_PLACE_REQS: R.PLACE_REQ, R.TABLE_DS: R.DS_REC,
+           R.TABLE_DS_ROLES: R.DS_ROLE_REC, R.TABLE_DS_REVROLES: R.DS_REVROLE_REC}
 
     # ----------------------------------------------------------- resident tick
     def resident_arena(self, min_bytes: int = 0) -> np.ndarray:
@@ -298,6 +302,14 @@ class Engine:
     def make_tick(self, segments=(), flags=0) -> "R.Tick":
         """Build a reusable ``lwse_tick`` descriptor.  ``segments``: (table, rows, values) with
         numpy arrays (ideally views of the arena), or (table, first_row, values, True) for a range."""
+        return self._fill_tick(R.Tick(), segments, flags)
+
+    def make_ds_tick(self, segments=()) -> "R.DsTick":
+        """A reusable ``lwse_ds_tick`` descriptor; ``segments`` as for ``make_tick`` (tables
+        ``TABLE_DS`` / ``TABLE_DS_ROLES`` / ``TABLE_DS_REVROLES``)."""
+        return self._fill_tick(R.DsTick(), segments, 0)
+
+    def _fill_tick(self, t, segments, flags):
         segs = (R.PatchSeg * max(len(segments), 1))()
         keep = []
         for i, sg in enumerate(segments):
@@ -311,7 +323,6 @@ class Engine:
                 segs[i] = R.PatchSeg(table, 0, len(rows), 0, R.ptr(rows) if len(rows) else None,
                                      R.ptr(values) if len(rows) else None)
                 keep.append((rows, values))
-        t = R.Tick()
         t.segs = segs
         t.n_segs = len(segments)
         t.flags = flags
@@ -462,6 +473,40 @@ class Engine:
             R.ptr(d_ds_out), R.ptr(d_role_out), R.ptr(d_revrole_out),
         )
         self._check(lib().lwse_sweep_ds_device(self._h, C.byref(t), stream))
+
+    def ds_resident_load(self, ds, roles, revroles):
+        """Make the three DS input tables resident on the device (committed results start at zero)."""
+        assert ds.dtype == R.DS_REC and roles.dtype == R.DS_ROLE_REC and revroles.dtype == R.DS_REVROLE_REC
+        self._ds_shape = (len(ds), len(roles), len(revroles))
+        t = R.DsTables(R.ptr(ds), len(ds), R.ptr(roles), len(roles), R.ptr(revroles), len(revroles), None, None, None)
+        self._check(lib().lwse_ds_resident_load(self._h, C.byref(t)))
+
+    def ds_resident_tick(self, tick: "R.DsTick"):
+        """One DS tick: patches in, listed result rows out → dict of numpy views of engine-owned
+        pinned memory (valid until the next resident call)."""
+        self._check(lib().lwse_ds_resident_tick(self._h, C.byref(tick)))
+
+        def view(ptr, n, dtype):
+            if not ptr or n == 0:
+                return np.zeros(0, dtype=dtype)
+            nbytes = n * np.dtype(dtype).itemsize
+            return np.frombuffer((C.c_uint8 * nbytes).from_address(ptr), dtype=dtype)
+
+        return {
+            "ds_rows": view(tick.ds_rows, tick.n_ds, np.uint32), "ds_out": view(tick.ds_out, tick.n_ds, R.DS_OUT),
+            "role_rows": view(tick.role_rows, tick.n_roles, np.uint32),
+            "role_out": view(tick.role_out, tick.n_roles, R.DS_ROLE_OUT),
+            "revrole_rows": view(tick.revrole_rows, tick.n_revroles, np.uint32),
+            "revrole_out": view(tick.revrole_out, tick.n_revroles, R.DS_REVROLE_OUT),
+            "n_ds": tick.n_ds, "n_roles": tick.n_roles, "n_revroles": tick.n_revroles,
+        }
+
+    def ds_resident_outputs(self):
+        """Every committed DS result row → (ds_out, role_out, revrole_out)."""
+        n_ds, n_ro, n_rr = self._ds_shape
+        o = (R.aligned_empty(n_ds, R.DS_OUT), R.aligned_empty(n_ro, R.DS_ROLE_OUT), R.aligned_empty(n_rr, R.DS_REVROLE_OUT))
+        self._check(lib().lwse_ds_resident_outputs(self._h, *(R.ptr(x) for x in o)))
+        return o
 
     # ------------------------------------------------------------- group keys
     def group_keys_host(self, strings) -> np.ndarray:

@@ -299,3 +299,148 @@ class IncrementalEncoder:
 
     def lws_row(self, namespace: str, name: str) -> int:
         return self.slots[(namespace, name)].lws_row
+
+
+# --------------------------------------------------------------------------- #
+# DisaggregatedSet controller: For(DisaggregatedSet), Owns(LeaderWorkerSet)
+# --------------------------------------------------------------------------- #
+@dataclass
+class DsSlots:
+    ds_row: int
+    role_base: int
+    role_cap: int
+    rev_base: int
+    rev_cap: int
+
+
+class DsIncrementalEncoder:
+    """The DS tables of ``lwse_ds_resident_tick`` kept current from the DS controller's watches
+    (disaggregatedset_controller.go:271-286: ``For(DisaggregatedSet)``, ``Owns(LeaderWorkerSet)``).
+
+    Laid out like ``IncrementalEncoder``: every DS owns a slot of role rows and of (revision, role)
+    rows with slack; ``flush()`` re-encodes the dirty DSes with ``encoder.encode_ds([item])`` and
+    emits one patch segment per table holding the rows that differ (the DS row included, when
+    ``n_roles`` / ``n_old_revs`` change); a DS that outgrows its slot moves to the spare rows at the
+    end of the tables, and when those run out ``needs_reload`` is set.  A DS ADDED / DELETED event
+    changes the DS table's shape: it sets ``needs_reload`` too.
+
+    Creation-timestamp ranks are per DS here (each DS is encoded on its own), not global as in one
+    ``encode_ds`` over every DS.  That is equivalent: ``sortByNewestTimestamp`` (executor.go:283-302)
+    only compares the revisions of one DS, and a per-DS rank preserves their order and ties.
+    """
+
+    def __init__(self, items: list, spare: float = 0.25):
+        self.items: dict[tuple, encoder.DsItem] = {(it.ds.namespace, it.ds.name): it for it in items}
+        self.needs_reload = False
+        self.dirty: set = set()
+        keys = sorted(self.items)
+        fresh = {k: encoder.encode_ds([self.items[k]]) for k in keys}
+        self.slots: dict[tuple, DsSlots] = {}
+        ro = rr = 0
+        for i, k in enumerate(keys):
+            t = fresh[k]
+            rcap, vcap = _slack(len(t.roles)), _slack(len(t.revroles))
+            self.slots[k] = DsSlots(i, ro, rcap, rr, vcap)
+            ro, rr = ro + rcap, rr + vcap
+        self.order = keys
+        self.ds = R.aligned_empty(len(keys), R.DS_REC)
+        self.roles = R.aligned_empty(ro + max(16, int(ro * spare)), R.DS_ROLE_REC)
+        self.revroles = R.aligned_empty(rr + max(64, int(rr * spare)), R.DS_REVROLE_REC)
+        self.role_end, self.rev_end = ro, rr
+        self._names: dict[tuple, list] = {}
+        self._old_revs: dict[tuple, list] = {}
+        for k in keys:
+            self._write(k, fresh[k], None)
+
+    # ------------------------------------------------------------------ layout
+    def _write(self, key, t: encoder.DsTablesHost, pending: Optional[dict]):
+        sl = self.slots[key]
+        if len(t.roles) > sl.role_cap or len(t.revroles) > sl.rev_cap:
+            rcap, vcap = _slack(len(t.roles)), _slack(len(t.revroles))
+            if self.role_end + rcap > len(self.roles) or self.rev_end + vcap > len(self.revroles):
+                self.needs_reload = True
+                return
+            sl = self.slots[key] = DsSlots(sl.ds_row, self.role_end, rcap, self.rev_end, vcap)
+            self.role_end, self.rev_end = self.role_end + rcap, self.rev_end + vcap
+        self._names[key], self._old_revs[key] = t.role_names[0], t.old_revisions[0]
+        row = t.ds.copy()
+        row["role_base"], row["rev_base"] = sl.role_base, sl.rev_base
+        for table_id, table, base, fresh_rows in ((R.TABLE_DS, self.ds, sl.ds_row, row),
+                                                  (R.TABLE_DS_ROLES, self.roles, sl.role_base, t.roles),
+                                                  (R.TABLE_DS_REVROLES, self.revroles, sl.rev_base, t.revroles)):
+            n = len(fresh_rows)
+            if n == 0:
+                continue
+            cur = table[base: base + n]
+            if pending is None:
+                cur[:] = fresh_rows
+                continue
+            a = np.ascontiguousarray(cur).view(np.uint8).reshape(n, -1)
+            b = np.ascontiguousarray(fresh_rows).view(np.uint8).reshape(n, -1)
+            diff = np.flatnonzero((a != b).any(axis=1))
+            if len(diff):
+                vals = R.aligned_empty(len(diff), table.dtype)
+                vals[:] = fresh_rows[diff]
+                cur[diff] = vals
+                rows, chunks = pending.setdefault(table_id, ([], []))
+                rows.extend((diff + base).tolist())
+                chunks.append(vals)
+
+    # ------------------------------------------------------------------ events
+    def ds_event(self, kind: str, item: encoder.DsItem):
+        """A watch event of the DisaggregatedSet informer.  MODIFIED (spec or target revision): the
+        children stay those the child events delivered.  ADDED / DELETED: reload."""
+        key = (item.ds.namespace, item.ds.name)
+        if kind != "MODIFIED" or key not in self.items:
+            self.needs_reload = True
+            return
+        self.items[key] = encoder.DsItem(item.ds, item.revision, self.items[key].children)
+        self.dirty.add(key)
+
+    def child_event(self, kind: str, ds_key: tuple, child: api.ChildLWS):
+        """A watch event of an owned LeaderWorkerSet (ADDED | MODIFIED | DELETED): replicas,
+        readyReplicas, annotations, or the child itself.  The List order (first seen) is kept."""
+        it = self.items.get(ds_key)
+        if it is None:
+            return
+        kids = it.children
+        at = next((i for i, c in enumerate(kids) if c.role == child.role and c.revision == child.revision), None)
+        if kind == "DELETED":
+            if at is not None:
+                kids.pop(at)
+        elif at is None:
+            kids.append(child)
+        else:
+            kids[at] = child
+        self.dirty.add(ds_key)
+
+    def flush(self) -> Patches:
+        """Re-encode the dirty DSes → the patch segments of one ``lwse_ds_resident_tick``."""
+        pending: dict = {}
+        for key in sorted(self.dirty):
+            self._write(key, encoder.encode_ds([self.items[key]]), pending)
+        self.dirty.clear()
+        patches = Patches()
+        for table_id in (R.TABLE_DS, R.TABLE_DS_ROLES, R.TABLE_DS_REVROLES):
+            if table_id in pending:
+                rows, chunks = pending[table_id]
+                patches.add(table_id, rows, np.concatenate(chunks))
+        return patches
+
+    # ------------------------------------------------------------------ results
+    def full_tables(self):
+        """(ds, roles, revroles): the whole allocation, spare rows included (what ``ds_resident_load``
+        takes, so that relocations stay in range)."""
+        return self.ds, self.roles, self.revroles
+
+    def ds_row(self, key) -> int:
+        return self.slots[key].ds_row
+
+    def role_names(self, key) -> list:
+        """allRoleNames of the DS: role i is row ``slots[key].role_base + i``."""
+        return self._names[key]
+
+    def old_revisions(self, key) -> list:
+        """Old revisions in row order: revision r, role i is row ``rev_base + r * n_roles + i``; the
+        target revision follows them (bit r of ``drained_revs`` / ``ready_revs`` is revision r)."""
+        return self._old_revs[key]

@@ -314,6 +314,7 @@ class Changes(C.Structure):
 
 
 TABLE_LWS, TABLE_GROUPS, TABLE_POD_STATE, TABLE_POD_IDENT, TABLE_PLACE_REQS = 0, 1, 2, 3, 4
+TABLE_DS, TABLE_DS_ROLES, TABLE_DS_REVROLES = 5, 6, 7  # the DS tick's tables (lwse_ds_resident_tick)
 PATCH_RANGE = 1 << 0
 TICK_MAX_SEGS = 8
 TICK_PLACE = 1 << 8
@@ -347,6 +348,24 @@ class Tick(C.Structure):
         ("place_out", C.c_void_p),
         ("n_place", C.c_uint32),
         ("place_rounds", C.c_uint32),
+    ]
+
+
+class DsTick(C.Structure):
+    _fields_ = [
+        ("segs", C.POINTER(PatchSeg)),
+        ("n_segs", C.c_uint32),
+        ("flags", C.c_uint32),
+        ("ds_rows", C.c_void_p),
+        ("ds_out", C.c_void_p),
+        ("n_ds", C.c_uint32),
+        ("n_roles", C.c_uint32),
+        ("role_rows", C.c_void_p),
+        ("role_out", C.c_void_p),
+        ("revrole_rows", C.c_void_p),
+        ("revrole_out", C.c_void_p),
+        ("n_revroles", C.c_uint32),
+        ("reserved", C.c_uint32),
     ]
 
 
