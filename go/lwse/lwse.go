@@ -155,6 +155,48 @@ func (e *Engine) DsTick(segs []C.lwse_patch_seg) (DsTickResult, error) {
 	}, nil
 }
 
+// JointSubmit enqueues one pass of both controllers (lwse_joint_tick_submit): the LWS part as Submit
+// (lwsSegs / flags; hasLws = false for a DS-only tick) and the DS
+// part as DsTick, one scatter, one publish.  It shares the two-slot ring of Submit; JointWait takes the
+// oldest tick of either kind (an LWS-only tick reports no DS rows).  The patch bytes of a submitted tick
+// stay untouched until its JointWait returned.  Uncompiled, like the rest of this file.
+func (e *Engine) JointSubmit(hasLws bool, lwsSegs []C.lwse_patch_seg, flags uint32, dsSegs []C.lwse_patch_seg) error {
+	var t C.lwse_tick
+	var d C.lwse_ds_tick
+	if len(lwsSegs) > 0 {
+		t.segs = (*C.lwse_patch_seg)(unsafe.Pointer(&lwsSegs[0]))
+		t.n_segs = C.uint32_t(len(lwsSegs))
+	}
+	t.flags = C.uint32_t(flags)
+	if len(dsSegs) > 0 {
+		d.segs = &dsSegs[0]
+		d.n_segs = C.uint32_t(len(dsSegs))
+	}
+	tp := &t
+	if !hasLws {
+		tp = nil
+	}
+	return e.check(C.lwse_joint_tick_submit(e.h, tp, &d))
+}
+
+// JointWait blocks for the oldest tick in flight → both controllers' listed rows (views valid until
+// the second submit after this call).
+func (e *Engine) JointWait() (TickResult, DsTickResult, error) {
+	var t C.lwse_tick
+	var d C.lwse_ds_tick
+	if err := e.check(C.lwse_joint_tick_wait(e.h, &t, &d)); err != nil {
+		return TickResult{}, DsTickResult{}, err
+	}
+	return tickResult(&t), DsTickResult{
+		DsRows:      unsafe.Slice((*uint32)(unsafe.Pointer(d.ds_rows)), int(d.n_ds)),
+		DsOut:       unsafe.Slice(d.ds_out, int(d.n_ds)),
+		RoleRows:    unsafe.Slice((*uint32)(unsafe.Pointer(d.role_rows)), int(d.n_roles)),
+		RoleOut:     unsafe.Slice(d.role_out, int(d.n_roles)),
+		RevroleRows: unsafe.Slice((*uint32)(unsafe.Pointer(d.revrole_rows)), int(d.n_revroles)),
+		RevroleOut:  unsafe.Slice(d.revrole_out, int(d.n_revroles)),
+	}, nil
+}
+
 // DsResidentOutputs copies every committed DS result row into the caller's tables (nil skips one).
 func (e *Engine) DsResidentOutputs(ds *C.lwse_ds_out, roles *C.lwse_ds_role_out, revroles *C.lwse_ds_revrole_out) error {
 	return e.check(C.lwse_ds_resident_outputs(e.h, ds, roles, revroles))

@@ -332,6 +332,8 @@ LWSE_API uint32_t lwse_abi_version(void);
 LWSE_API void* lwse_stream(const lwse_engine* e);
 /* Number of kernels this engine has launched since creation. */
 LWSE_API uint64_t lwse_launch_count(const lwse_engine* e);
+/* Number of resident ticks this engine has replayed as one CUDA graph (LWSE_TICK_GRAPH) since creation. */
+LWSE_API uint64_t lwse_graph_tick_count(const lwse_engine* e);
 
 /* Shard an object onto one of n engines (Go: hash(LWS.UID) mod nGPU; DS-owned
  * LWS pass the DS uid hash so a DS and its children co-reside). */
@@ -734,14 +736,16 @@ LWSE_API int lwse_sweep_ds_device(lwse_engine* e, const lwse_ds_tables* dev_tabl
  * Invariant: a zero mirror with every tick's lists applied in order equals lwse_ds_resident_outputs
  * on every row (and, on the rows valid DSes own, the stateless sweep of the same tables).
  * Like every other resident call, a DS resident call first waits for (and drops the results of) the
- * LWS ticks in flight.  One DS tick runs at a time. */
+ * ticks in flight.  One DS tick runs at a time; to keep two in flight, use the joint tick below with
+ * lws = NULL. */
 typedef struct lwse_ds_tick {
   /* in */
   const lwse_patch_seg* segs; /* tables LWSE_TABLE_DS .. LWSE_TABLE_DS_REVROLES only */
   uint32_t n_segs;            /* <= LWSE_TICK_MAX_SEGS */
   uint32_t flags;             /* reserved, 0 */
   /* out: views of engine-owned pinned memory, valid until the next lwse_*resident* call on this
-   * engine.  n_* counts the listed rows (at most the table's rows).  Order is unspecified. */
+   * engine (joint ticks: see lwse_joint_tick).  n_* counts the listed rows (at most the table's rows).
+   * Order is unspecified. */
   const uint32_t* ds_rows;
   const lwse_ds_out* ds_out;
   uint32_t n_ds;
@@ -761,6 +765,44 @@ LWSE_API int lwse_ds_resident_tick(lwse_engine* e, lwse_ds_tick* t);
 /* Every committed result row (n_ds / n_roles / n_revroles rows of the loaded tables; NULL skips). */
 LWSE_API int lwse_ds_resident_outputs(lwse_engine* e, lwse_ds_out* ds_out, lwse_ds_role_out* role_out,
                                       lwse_ds_revrole_out* revrole_out);
+
+/* ---- the joint tick: one pass of the LWS, pod and DS controllers' work queues, one call ----------
+ * One tick of both controllers: the LWS part exactly as lwse_resident_tick_submit, the DS part with the
+ * listing rules of lwse_ds_resident_tick, ONE scatter, ONE publish.  lws may be NULL (a DS-only tick,
+ * which pipelines like an LWS tick); ds may not.
+ *   patches of both parts -> scatter kernel -> fused pod scan + group pass -> LWS pass ---> publish
+ *                                           \-> DS sweep (own stream) -------------------/
+ *                         \-> placement round (side stream) --------------------------/
+ * Rules:
+ *   - Preconditions: lwse_ds_resident_load, else LWSE_ERR_NOT_READY; lwse_resident_load when lws != NULL,
+ *     and lwse_resident_place_load when lws->flags has LWSE_TICK_PLACE (else LWSE_ERR_NOT_READY).  An
+ *     engine with DS tables only runs DS-only joint ticks.
+ *   - lws->segs name tables 0-4 only, ds->segs tables 5-7 only, at most LWSE_TICK_MAX_SEGS each;
+ *     ds->flags must be 0; LWSE_TICK_SHARED_OCCUPANCY is refused (LWSE_ERR_INVALID_ARG): a joint tick
+ *     runs on one rank.
+ *   - A refused call does nothing: it enqueues nothing, takes no ring slot, moves no sequence number.
+ *   - One ring: joint ticks share the two slots of lwse_resident_tick_submit.  At most two ticks of
+ *     either kind are in flight; a third submit returns LWSE_ERR_NOT_READY.
+ *   - lwse_joint_tick_wait takes the oldest tick of either kind (lws may be NULL: its LWS results are
+ *     then not reported); for an LWS-only tick it fills ds with zero counts and NULL views.
+ *     lwse_resident_tick_wait refuses a joint tick at the head of the ring (LWSE_ERR_INVALID_ARG) and
+ *     leaves it in flight, so its DS lists are not lost.
+ *   - lwse_joint_tick == _submit + _wait of one tick; with ticks in flight it returns LWSE_ERR_NOT_READY
+ *     (their results stay with _wait).
+ *   - Output views (both parts) and arena regions have the lifetime of lwse_resident_tick_submit's:
+ *     views stay valid until the second submit after their wait, patch segments stay untouched until
+ *     their wait returned.
+ *   - Every other resident call (lwse_ds_resident_tick, lwse_ds_resident_load, lwse_resident_load, ...)
+ *     still first waits for (and drops the results of) the ticks in flight.  Joint ticks and
+ *     lwse_ds_resident_tick share the DS committed outputs: the committed-value model above applies
+ *     across both.
+ *   - The DS change lists follow committed values exactly as in lwse_ds_resident_tick, in stream order
+ *     across pipelined ticks: a zero mirror with every tick's lists applied in order equals
+ *     lwse_ds_resident_outputs.
+ *   - A joint tick is enqueued kernel by kernel (LWSE_TICK_GRAPH does not apply to it). */
+LWSE_API int lwse_joint_tick(lwse_engine* e, lwse_tick* lws, lwse_ds_tick* ds);
+LWSE_API int lwse_joint_tick_submit(lwse_engine* e, const lwse_tick* lws, const lwse_ds_tick* ds);
+LWSE_API int lwse_joint_tick_wait(lwse_engine* e, lwse_tick* lws, lwse_ds_tick* ds);
 
 /* ------------------------------------------------------------------------- */
 /* Group / subgroup keys (SHA-1) and subgroup indices                        */

@@ -227,3 +227,65 @@ def apply_ds_to_mirror(ps: DsPatchSet, roles: np.ndarray, revroles: np.ndarray) 
     revroles[ps.rr_rows] = ps.rr_vals
     if len(ps.role_rows):
         roles[ps.role_rows] = ps.role_vals
+
+
+# --------------------------------------------------------------------------- #
+# Joint LWS + DS ticks (lwse_joint_tick_submit)
+# --------------------------------------------------------------------------- #
+def _arena_bytes(arrays) -> int:
+    return sum((a.nbytes + 255) // 256 * 256 for a in arrays)
+
+
+class JointArenaPlan:
+    """The joint counterpart of ``ArenaPlan``: pass k's LWS ``PatchSet`` and ``DsPatchSet`` are
+    written into region k % 2 of the engine's patch arena, so that two joint ticks can be in flight.
+    Pass k+2 reuses the region of pass k: submit it only after pass k's wait returned (the engine
+    allows two ticks in flight, so a pipelined caller has waited for it by then).  ``lws_sets``
+    None: DS-only ticks.  Every array starts on a 256-byte boundary of its region."""
+
+    def __init__(self, engine, lws_sets, ds_sets, flags: int = 0):
+        self.engine, self.lws_sets, self.ds_sets, self.flags = engine, lws_sets, ds_sets, flags
+        self.n_passes = len(ds_sets)
+        assert lws_sets is None or len(lws_sets) == self.n_passes
+        need = max((_arena_bytes(self._arrays(k)) for k in range(self.n_passes)), default=0)
+        self.region_bytes = (need + 4095) // 4096 * 4096
+        self.arena = engine.resident_arena(2 * self.region_bytes)
+        self.spans = []  # (pass, byte offset, bytes) of every array tick() wrote, in order
+
+    def _arrays(self, k):
+        out = []
+        if self.lws_sets is not None:
+            ps = self.lws_sets[k]
+            out += [a for pair in ((ps.pod_rows, ps.pod_vals), (ps.grp_rows, ps.grp_vals), (ps.req_rows, ps.req_vals))
+                    if len(pair[0]) for a in pair]
+        d = self.ds_sets[k]
+        out += [a for pair in ((d.rr_rows, d.rr_vals), (d.role_rows, d.role_vals)) if len(pair[0]) for a in pair]
+        return out
+
+    def tick(self, k: int):
+        """Write pass k % n_passes into its region → (Tick or None, DsTick) descriptors pointing there."""
+        p = k % self.n_passes
+        cursor = (k % 2) * self.region_bytes
+
+        def put(a):
+            nonlocal cursor
+            view = self.arena[cursor: cursor + a.nbytes].view(a.dtype)
+            view[...] = a.reshape(-1) if a.dtype.fields is None else a
+            self.spans.append((k, cursor, a.nbytes))
+            cursor += (a.nbytes + 255) // 256 * 256
+            return view
+
+        lws_tick = None
+        if self.lws_sets is not None:
+            ps, segs = self.lws_sets[p], []
+            for table, rows, vals in ((R.TABLE_POD_STATE, ps.pod_rows, ps.pod_vals), (R.TABLE_GROUPS, ps.grp_rows, ps.grp_vals),
+                                      (R.TABLE_PLACE_REQS, ps.req_rows, ps.req_vals)):
+                if len(rows):
+                    segs.append((table, put(rows), put(vals)))
+            lws_tick = self.engine.make_tick(segs, self.flags)
+        d, segs = self.ds_sets[p], []
+        for table, rows, vals in ((R.TABLE_DS_REVROLES, d.rr_rows, d.rr_vals), (R.TABLE_DS_ROLES, d.role_rows, d.role_vals)):
+            if len(rows):
+                segs.append((table, put(rows), put(vals)))
+        assert cursor <= (k % 2 + 1) * self.region_bytes
+        return lws_tick, self.engine.make_ds_tick(segs)

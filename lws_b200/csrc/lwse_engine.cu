@@ -38,6 +38,9 @@ struct PublishListHost {
 int launch_publish(const PublishListHost* lists, const uint32_t* d_extra, uint32_t* h_words, uint32_t seq_slot,
                    uint32_t seq, uint32_t* d_ticket, uint32_t expected_rows, cudaStream_t s, int* cuda_err,
                    uint32_t* d_clear, uint32_t n_clear, bool pdl);
+int launch_publish_joint(const PublishListHost* lists, const uint32_t* d_extra, uint32_t* h_words, uint32_t seq_slot,
+                         uint32_t seq, uint32_t* d_ticket, uint32_t expected_rows, cudaStream_t s, int* cuda_err,
+                         uint32_t* d_clear, uint32_t n_clear);
 cudaError_t set_sweep_carveout(int pct);
 cudaError_t set_place_ns_carveout(int pct);
 int launch_lws_sweep(const lwse_lws_tables* t, const lwse_node_rec* d_nodes, uint32_t n_nodes,
@@ -225,7 +228,8 @@ struct lwse_engine {
   PinBuf chg;                        // change lists: [lws rows | lws out | group rows | group out | place rows | place out]
   DevBuf chg_dev;                    // the same layout in device memory: the kernels append here, a publish kernel copies out
   uint32_t last_changed[2] = {0, 0}; // rows the previous tick reported (sweep lists, placement list): sizes the publish grid
-  PinBuf tickw;                      // [0] lws changes [1] group changes [2] place changes [3] placement rounds [4] sequence word
+  PinBuf tickw;                      // per tick slot (16 words): [0] lws changes [1] group changes [2] place changes
+                                     // [3] placement rounds [4] sequence word; a joint tick also [5] ds [6] role [7] revrole
   size_t chg_off[6] = {};
   uint32_t rn_lws = 0, rn_groups = 0, rn_reqs = 0, rn_namespaces = 0;
   uint64_t rn_pods = 0;
@@ -235,6 +239,7 @@ struct lwse_engine {
   struct TickSlot {
     uint32_t seq = 0;
     bool do_sweep = false, do_place = false, published = false, wrote = false;
+    bool joint = false;  // lwse_joint_tick_submit: the slot's DS lists are published too
   } tslot[2];
   uint64_t t_submitted = 0, t_waited = 0;
   size_t chg_bytes = 0;              // one slot of `chg`
@@ -259,6 +264,8 @@ struct lwse_engine {
   int use_graph = 1;                 // LWSE_TICK_GRAPH: 0 never, 1 when a tick is in flight (default), 2 always
   uint64_t graph_ticks = 0;
   cudaEvent_t ev_pub = nullptr;      // behind the previous tick's publish kernel: the next tick's side stream starts there
+  cudaStream_t ds_stream = nullptr;   // a joint tick's DS sweep: forked behind the scatter, joined before the publish
+  cudaEvent_t ev_ds_fork = nullptr, ev_ds_join = nullptr;
   int tick_order = 0;                // LWSE_TICK_ORDER (A/B of the tick's enqueue order, see tick_locked)
   uint32_t* h_counts = nullptr;      // pinned, 2 words
   DevBuf h_counts_dev;               // event-pod count of the host entry point's sweep
@@ -281,11 +288,13 @@ struct lwse_engine {
   // resident DS tables (lwse_ds_resident_*): inputs, committed outputs, scratch, change lists — none
   // shared with the stateless DS sweep's staging above or with the LWS resident state
   DevBuf rd_ds, rd_roles, rd_revroles, rd_ds_out, rd_role_out, rd_revrole_out, rd_role_scratch, rd_revrole_scratch;
+  // Change lists and counters per tick slot: a joint tick uses the ring slot it takes, lwse_ds_resident_tick slot 0.
   DevBuf rd_chg_dev;                 // change lists: [ds rows | ds out | role rows | role out | revrole rows | revrole out]
-  DevBuf rd_counts;                  // [0] ds [1] role [2] revrole rows listed, [3] publish ticket
+  DevBuf rd_counts;                  // 16 words per slot: [0] ds [1] role [2] revrole rows listed, [3] publish ticket
   PinBuf rd_chg;                     // the same layout in pinned, mapped memory (the publish kernel copies into it)
-  PinBuf rd_tickw;                   // [0..2] the three counts, [4] sequence word
+  PinBuf rd_tickw;                   // lwse_ds_resident_tick: [0..2] the three counts, [4] sequence word
   size_t rd_chg_off[6] = {};
+  size_t rd_chg_bytes = 0;           // one slot of rd_chg / rd_chg_dev
   uint32_t rdn_ds = 0, rdn_roles = 0, rdn_revroles = 0;
   uint32_t rd_seq = 0, rd_last_changed = 0;
   bool rd_loaded = false, rd_first = false;
@@ -458,6 +467,13 @@ LWSE_API int lwse_create(const lwse_config* cfg, lwse_engine** out) {
     lwse_destroy(e);
     return LWSE_ERR_OOM;
   }
+  if (cudaStreamCreateWithFlags(&e->ds_stream, cudaStreamNonBlocking) != cudaSuccess ||
+      cudaEventCreateWithFlags(&e->ev_ds_fork, cudaEventDisableTiming) != cudaSuccess ||
+      cudaEventCreateWithFlags(&e->ev_ds_join, cudaEventDisableTiming) != cudaSuccess) {
+    (void)cudaGetLastError();
+    lwse_destroy(e);
+    return LWSE_ERR_CUDA;
+  }
   {
     const char* v = getenv("LWSE_NO_ZERO_COPY");
     e->no_zero_copy = v && atoi(v) != 0;
@@ -519,6 +535,12 @@ LWSE_API void lwse_destroy(lwse_engine* e) {
     if (e->ev_done) cudaEventDestroy(e->ev_done);
     if (e->ev_mid) cudaEventDestroy(e->ev_mid);
     if (e->pub_stream) cudaStreamDestroy(e->pub_stream);
+    if (e->ds_stream) {
+      cudaStreamSynchronize(e->ds_stream);
+      cudaStreamDestroy(e->ds_stream);
+    }
+    if (e->ev_ds_fork) cudaEventDestroy(e->ev_ds_fork);
+    if (e->ev_ds_join) cudaEventDestroy(e->ev_ds_join);
     cudaStreamDestroy(e->side_stream);
     cudaStreamDestroy(e->stream);
   }
@@ -528,6 +550,7 @@ LWSE_API void lwse_destroy(lwse_engine* e) {
 LWSE_API int lwse_last_cuda_error(const lwse_engine* e) { return e ? e->last_cuda_error : 0; }
 LWSE_API void* lwse_stream(const lwse_engine* e) { return e ? (void*)e->stream : nullptr; }
 LWSE_API uint64_t lwse_launch_count(const lwse_engine* e) { return e ? e->launches : 0; }
+LWSE_API uint64_t lwse_graph_tick_count(const lwse_engine* e) { return e ? e->graph_ticks : 0; }
 
 LWSE_API int lwse_upload_nodes(lwse_engine* e, const lwse_node_rec* nodes, uint32_t n_nodes,
                                uint32_t n_domains) {
@@ -810,19 +833,18 @@ LWSE_API int lwse_resident_arena(lwse_engine* e, uint64_t min_bytes, void** base
   return LWSE_OK;
 }
 
-// table → (device base, rows, bytes per row).  `ds`: the tables of the DS tick (ids 5-7), which the
-// LWS tick does not take; the DS tick takes nothing else.
-static bool resident_table(lwse_engine* e, uint32_t which, void** base, uint64_t* rows, uint32_t* row_bytes, bool ds = false) {
-  if (ds) {
-    switch (which) {
-      case LWSE_TABLE_DS: *base = e->rd_ds.p; *rows = e->rdn_ds; *row_bytes = sizeof(lwse_ds_rec); return true;
-      case LWSE_TABLE_DS_ROLES: *base = e->rd_roles.p; *rows = e->rdn_roles; *row_bytes = sizeof(lwse_ds_role_rec); return true;
-      case LWSE_TABLE_DS_REVROLES:
-        *base = e->rd_revroles.p; *rows = e->rdn_revroles; *row_bytes = sizeof(lwse_ds_revrole_rec); return true;
-      default: return false;
-    }
-  }
+// Table-id sets a call resolves: the LWS tick takes ids 0-4, the DS tick 5-7, a joint tick both.
+constexpr uint32_t kLwsTableIds = 0x1Fu, kDsTableIds = 0xE0u, kAllTableIds = kLwsTableIds | kDsTableIds;
+
+// table → (device base, rows, bytes per row); false for an id outside `ids`.
+static bool resident_table(lwse_engine* e, uint32_t which, void** base, uint64_t* rows, uint32_t* row_bytes,
+                           uint32_t ids = kLwsTableIds) {
+  if (which > LWSE_TABLE_DS_REVROLES || !((ids >> which) & 1u)) return false;
   switch (which) {
+    case LWSE_TABLE_DS: *base = e->rd_ds.p; *rows = e->rdn_ds; *row_bytes = sizeof(lwse_ds_rec); return true;
+    case LWSE_TABLE_DS_ROLES: *base = e->rd_roles.p; *rows = e->rdn_roles; *row_bytes = sizeof(lwse_ds_role_rec); return true;
+    case LWSE_TABLE_DS_REVROLES:
+      *base = e->rd_revroles.p; *rows = e->rdn_revroles; *row_bytes = sizeof(lwse_ds_revrole_rec); return true;
     case LWSE_TABLE_LWS: *base = e->r_lws.p; *rows = e->rn_lws; *row_bytes = sizeof(lwse_lws_rec); return true;
     case LWSE_TABLE_GROUPS: *base = e->r_groups.p; *rows = e->rn_groups; *row_bytes = sizeof(lwse_group_rec); return true;
     case LWSE_TABLE_POD_STATE: *base = e->r_pst.p; *rows = e->rn_pods; *row_bytes = sizeof(lwse_pod_state); return true;
@@ -851,7 +873,7 @@ static bool values_in_place(const lwse_engine* e, const lwse_patch_seg& g, uint3
 // patches on the side stream, where the round that reads them runs, and the rest on the engine's
 // stream); `stage_base`: where in the staging buffer this call may put copies.
 struct ScatterPlan {  // a prepared scatter launch (apply_patches_locked with `defer`): the copy is enqueued, the kernel is not
-  lwse::ScatterSegHost sc[LWSE_TICK_MAX_SEGS];
+  lwse::ScatterSegHost sc[2 * LWSE_TICK_MAX_SEGS];  // (both parts of a joint tick)
   int n = 0;
   bool recount = false;
   // with `plan_only`: nothing was enqueued at all; the arena span [lo, hi) still has to be copied
@@ -860,10 +882,13 @@ struct ScatterPlan {  // a prepared scatter launch (apply_patches_locked with `d
   size_t lo = 0, hi = 0;
 };
 
+// One scatter launch per LWSE_TICK_MAX_SEGS segments (the kernel's limit): only a joint tick can need a
+// second one, which follows programmatically and waits for the first at its top.
 static int launch_scatter_plan(lwse_engine* e, const ScatterPlan& p, cudaStream_t s) {
   int cuda_err = 0;
-  if (p.n) {
-    int launched = lwse::launch_scatter(p.sc, p.n, e->n_nodes ? (uint32_t*)e->r_occ.p : nullptr, e->n_nodes, s, true, &cuda_err);
+  for (int k0 = 0; k0 < p.n; k0 += (int)LWSE_TICK_MAX_SEGS) {
+    const int n = p.n - k0 < (int)LWSE_TICK_MAX_SEGS ? p.n - k0 : (int)LWSE_TICK_MAX_SEGS;
+    int launched = lwse::launch_scatter(p.sc + k0, n, e->n_nodes ? (uint32_t*)e->r_occ.p : nullptr, e->n_nodes, s, true, &cuda_err);
     if (launched < 0) return fail_cuda(e, (cudaError_t)cuda_err);
     e->launches += (uint64_t)launched;
   }
@@ -879,11 +904,12 @@ static int launch_scatter_plan(lwse_engine* e, const ScatterPlan& p, cudaStream_
 static int apply_patches_locked(lwse_engine* e, const lwse_patch_seg* segs, uint32_t n_segs, bool* wrote,
                                 uint32_t tables = 0xFFFFFFFFu, cudaStream_t s = nullptr, size_t stage_base = 0,
                                 size_t* stage_used = nullptr, long dma_min_bytes = 0, ScatterPlan* defer = nullptr,
-                                bool plan_only = false, bool ds = false) {
+                                bool plan_only = false, uint32_t ids = kLwsTableIds) {
   *wrote = false;
   if (stage_used) *stage_used = stage_base;
   if (n_segs == 0) return LWSE_OK;
-  if (!segs || n_segs > LWSE_TICK_MAX_SEGS) return LWSE_ERR_INVALID_ARG;
+  // (a joint tick hands both parts' segments in one call, each part at most LWSE_TICK_MAX_SEGS)
+  if (!segs || n_segs > (ids == kAllTableIds ? 2u : 1u) * LWSE_TICK_MAX_SEGS) return LWSE_ERR_INVALID_ARG;
   if (!s) s = e->stream;
   // room for every segment that is not in the arena
   size_t need = 0;
@@ -891,7 +917,7 @@ static int apply_patches_locked(lwse_engine* e, const lwse_patch_seg* segs, uint
     void* base;
     uint64_t rows;
     uint32_t rb;
-    if (!resident_table(e, segs[i].table, &base, &rows, &rb, ds)) return LWSE_ERR_INVALID_ARG;
+    if (!resident_table(e, segs[i].table, &base, &rows, &rb, ids)) return LWSE_ERR_INVALID_ARG;
     if (segs[i].n == 0 || !((tables >> segs[i].table) & 1u)) continue;
     if (!segs[i].values || (!(segs[i].flags & LWSE_PATCH_RANGE) && !segs[i].rows)) return LWSE_ERR_INVALID_ARG;
     if (segs[i].flags & LWSE_PATCH_RANGE) {
@@ -918,7 +944,7 @@ static int apply_patches_locked(lwse_engine* e, const lwse_patch_seg* segs, uint
     void* base;
     uint64_t rows;
     uint32_t rb;
-    resident_table(e, g.table, &base, &rows, &rb, ds);
+    resident_table(e, g.table, &base, &rows, &rb, ids);
     *wrote = true;
     if (g.table == LWSE_TABLE_PLACE_REQS && e->r_place_grouped) {
       // a request that moves to another namespace breaks the grouping the fast placement kernels rely on
@@ -1583,14 +1609,20 @@ static bool wait_word(volatile uint32_t* w, uint32_t seq, cudaStream_t s, cudaEr
 
 struct TickCounts {
   uint32_t n_lws = 0, n_groups = 0, n_place = 0, rounds = 0;
+  uint32_t n_ds = 0, n_roles = 0, n_revroles = 0;  // a joint tick's DS lists
 };
+
+static int enqueue_ds_sweep(lwse_engine* e, uint32_t slot, bool first, cudaStream_t s, bool pdl, lwse::PublishListHost* pl,
+                            int* launched_out);
 
 static inline uint8_t* d_desc_of(lwse_engine* e, uint32_t slot, size_t desc_bytes) {
   return static_cast<uint8_t*>(e->tdesc_dev.p) + slot * desc_bytes;
 }
 
 // Enqueue one tick (nothing waits): slot = t_submitted & 1.  At most two ticks are in flight.
-static int tick_submit_locked(lwse_engine* e, const lwse_patch_seg* segs, uint32_t n_segs, uint32_t flags) {
+// `joint` (lwse_joint_tick_submit): segs holds both parts' segments (table ids 0-7, checked by the caller) and the
+// resident DS sweep runs in the tick as well; its three lists are published with the tick's.
+static int tick_submit_locked(lwse_engine* e, const lwse_patch_seg* segs, uint32_t n_segs, uint32_t flags, bool joint = false) {
   if (e->t_submitted - e->t_waited >= 2) return LWSE_ERR_NOT_READY;  // wait for the oldest tick first
   const bool in_flight = e->t_submitted != e->t_waited;
   const uint32_t slot = (uint32_t)(e->t_submitted & 1u);
@@ -1603,8 +1635,10 @@ static int tick_submit_locked(lwse_engine* e, const lwse_patch_seg* segs, uint32
   const bool do_sweep = !(flags & LWSE_TICK_NO_SWEEP) && (e->rn_lws || e->rn_groups);
   if (n_segs && !segs) return LWSE_ERR_INVALID_ARG;
   // sequence numbers count the ticks that end in a publish kernel (the device counts the same ones)
+  const uint32_t ids = joint ? kAllTableIds : kLwsTableIds;
+  const bool ds_first = joint && e->rd_first;  // the first DS tick after lwse_ds_resident_load lists every row
   uint32_t seq = 0;
-  if (do_sweep || do_place) {
+  if (do_sweep || do_place || joint) {
     seq = ++e->tick_seq;
     if (seq == 0) seq = ++e->tick_seq;
   }
@@ -1653,7 +1687,7 @@ static int tick_submit_locked(lwse_engine* e, const lwse_patch_seg* segs, uint32
     void* tb;
     uint64_t trows;
     uint32_t rb = 0;
-    if (!resident_table(e, segs[i].table, &tb, &trows, &rb)) return LWSE_ERR_INVALID_ARG;
+    if (!resident_table(e, segs[i].table, &tb, &trows, &rb, ids)) return LWSE_ERR_INVALID_ARG;
     if (!rows_in_place(e, segs[i]) || !values_in_place(e, segs[i], rb)) all_in_place = false;
   }
   int order = has_ident ? 2 : e->tick_order;
@@ -1674,7 +1708,8 @@ static int tick_submit_locked(lwse_engine* e, const lwse_patch_seg* segs, uint32
   }
   ScatterPlan main_plan;
   auto apply_main = [&](bool defer) -> int {
-    return apply_patches_locked(e, segs, n_segs, &wrote, ~kSideTables, s, 0, &stage_used, 0, defer ? &main_plan : nullptr);
+    return apply_patches_locked(e, segs, n_segs, &wrote, ~kSideTables, s, 0, &stage_used, 0, defer ? &main_plan : nullptr, false,
+                                ids);
   };
   auto apply_side = [&]() -> int {
     if (has_ident && wrote && (has_side || do_place)) {
@@ -1682,9 +1717,10 @@ static int tick_submit_locked(lwse_engine* e, const lwse_patch_seg* segs, uint32
       LWSE_CUDA(e, cudaStreamWaitEvent(ps, e->ev_fork, 0));
     }
     if (!has_side) return LWSE_OK;
-    return apply_patches_locked(e, segs, n_segs, &wrote_side, kSideTables, ps, stage_used, nullptr, /*dma_min_bytes=*/65536);
+    return apply_patches_locked(e, segs, n_segs, &wrote_side, kSideTables, ps, stage_used, nullptr, /*dma_min_bytes=*/65536, nullptr,
+                                false, ids);
   };
-  lwse::PublishListHost pl[3] = {};
+  lwse::PublishListHost pl[6] = {};  // [0..2] the LWS tick's lists, [3..5] a joint tick's DS lists
   int sweep_first_mode = -1;      // -1: 2 behind this tick's scatter kernel, else 1 (see launch_lws_sweep)
   bool place_first_pdl = true;    // the round's first kernel follows a kernel on the side stream
   void* place_mid_event = nullptr;  // (graph capture) recorded between the condense and the namespace kernel
@@ -1755,9 +1791,12 @@ static int tick_submit_locked(lwse_engine* e, const lwse_patch_seg* segs, uint32
     LWSE_CUDA(e, cudaEventRecord(e->ev_done, s));
     LWSE_CUDA(e, cudaStreamWaitEvent(e->pub_stream, e->ev_done, 0));
     const bool ns_counters = do_place && e->tick_place_ns;
-    int launched = lwse::launch_publish(pl, do_place ? e->place_rounds_ptr : nullptr, hw_dev, 4, seq, cnt + 2,
-                                        e->last_changed[0] + e->last_changed[1], e->pub_stream, &cuda_err,
-                                        ns_counters ? const_cast<uint32_t*>(e->place_rounds_ptr) : nullptr, 8u, /*pdl=*/false);
+    int launched = joint ? lwse::launch_publish_joint(pl, do_place ? e->place_rounds_ptr : nullptr, hw_dev, 4, seq, cnt + 2,
+                                                      e->last_changed[0] + e->last_changed[1], e->pub_stream, &cuda_err,
+                                                      ns_counters ? const_cast<uint32_t*>(e->place_rounds_ptr) : nullptr, 8u)
+                         : lwse::launch_publish(pl, do_place ? e->place_rounds_ptr : nullptr, hw_dev, 4, seq, cnt + 2,
+                                                e->last_changed[0] + e->last_changed[1], e->pub_stream, &cuda_err,
+                                                ns_counters ? const_cast<uint32_t*>(e->place_rounds_ptr) : nullptr, 8u, /*pdl=*/false);
     if (launched < 0) return fail_cuda(e, (cudaError_t)cuda_err);
     e->launches += (uint64_t)launched;
     LWSE_CUDA(e, cudaEventRecord(e->ev_pub, e->pub_stream));
@@ -1779,7 +1818,7 @@ static int tick_submit_locked(lwse_engine* e, const lwse_patch_seg* segs, uint32
   //  host's enqueue time is what limits the rate; a lone tick is faster kernel by kernel, because its
   //  round starts while the copy engine still moves the pod patches; 2 = always; 0 = never)
   const bool shared_occ = (flags & LWSE_TICK_SHARED_OCCUPANCY) != 0;
-  const bool graph_ok = (e->use_graph >= 2 || (e->use_graph == 1 && in_flight)) && all_in_place && !any_range &&
+  const bool graph_ok = !joint && (e->use_graph >= 2 || (e->use_graph == 1 && in_flight)) && all_in_place && !any_range &&
                         (!shared_occ || (do_place && e->xch_connected)) &&
                         (do_sweep || do_place) && !(has_side && !do_place) &&
                         (!do_place || (e->r_place_grouped && g_place_form_env != 0 && lwse::place_ns_supported(e->n_nodes, e->n_domains)));
@@ -1906,35 +1945,53 @@ static int tick_submit_locked(lwse_engine* e, const lwse_patch_seg* segs, uint32
       gts.do_place = do_place;
       gts.published = true;
       gts.wrote = has_patches;
+      gts.joint = false;
       e->t_submitted++;
       return LWSE_OK;
     }
   }
+  // A joint tick's DS sweep reads only the DS tables, which only the main scatter writes: it forks behind
+  // the scatter onto its own stream and overlaps the LWS sweep; the publish waits for it.  (On its own
+  // stream it measured 100 us per serial C3 + C4 pass against 114 us behind the LWS pass; DESIGN §4.)
+  auto fork_ds = [&]() -> int {
+    if (!joint) return LWSE_OK;
+    LWSE_CUDA(e, cudaEventRecord(e->ev_ds_fork, s));
+    LWSE_CUDA(e, cudaStreamWaitEvent(e->ds_stream, e->ev_ds_fork, 0));
+    int n = 0;
+    const int r = enqueue_ds_sweep(e, slot, ds_first, e->ds_stream, false, pl + 3, &n);
+    if (r != LWSE_OK) return r;
+    LWSE_CUDA(e, cudaEventRecord(e->ev_ds_join, e->ds_stream));
+    return LWSE_OK;
+  };
   if (order == 1) {
     rc = apply_side();
     if (rc == LWSE_OK && do_place) rc = enqueue_place();
     if (rc == LWSE_OK) rc = apply_main(false);
+    if (rc == LWSE_OK) rc = fork_ds();
     if (rc == LWSE_OK && do_sweep) rc = enqueue_sweep();
   } else if (order == 0) {
     rc = apply_main(true);
     if (rc == LWSE_OK) rc = apply_side();
     if (rc == LWSE_OK && do_place && wrote) rc = enqueue_place();
     if (rc == LWSE_OK) rc = launch_scatter_plan(e, main_plan, s);
+    if (rc == LWSE_OK) rc = fork_ds();
     if (rc == LWSE_OK && do_sweep) rc = enqueue_sweep();
     if (rc == LWSE_OK && do_place && !wrote) rc = enqueue_place();
   } else {
     rc = apply_main(false);
+    if (rc == LWSE_OK) rc = fork_ds();
     if (rc == LWSE_OK) rc = apply_side();
     if (rc == LWSE_OK && do_place && wrote) rc = enqueue_place();
     if (rc == LWSE_OK && do_sweep) rc = enqueue_sweep();
     if (rc == LWSE_OK && do_place && !wrote) rc = enqueue_place();
   }
+  if (rc == LWSE_OK && joint) LWSE_CUDA(e, cudaStreamWaitEvent(s, e->ev_ds_join, 0));
   if (rc != LWSE_OK) return rc;
   if (do_place || wrote_side) {
     LWSE_CUDA(e, cudaEventRecord(e->ev_join, ps));
     LWSE_CUDA(e, cudaStreamWaitEvent(s, e->ev_join, 0));
   }
-  const bool published = do_sweep || do_place;
+  const bool published = do_sweep || do_place || joint;
   if (published) {
     rc = enqueue_publish();
     if (rc != LWSE_OK) return rc;
@@ -1945,6 +2002,8 @@ static int tick_submit_locked(lwse_engine* e, const lwse_patch_seg* segs, uint32
   ts.do_place = do_place;
   ts.published = published;
   ts.wrote = wrote || wrote_side;
+  ts.joint = joint;
+  if (joint) e->rd_first = false;
   e->t_submitted++;
   return LWSE_OK;
 }
@@ -1975,7 +2034,11 @@ static int tick_wait_locked(lwse_engine* e, TickCounts* out, uint32_t* slot_out)
   out->n_groups = ts.do_sweep ? hw[1] : 0u;
   out->n_place = ts.do_place ? hw[2] : 0u;
   out->rounds = ts.do_place ? hw[3] : 0u;
-  e->last_changed[0] = out->n_lws + out->n_groups;
+  out->n_ds = ts.joint ? hw[5] : 0u;
+  out->n_roles = ts.joint ? hw[6] : 0u;
+  out->n_revroles = ts.joint ? hw[7] : 0u;
+  e->last_changed[0] = out->n_lws + out->n_groups + out->n_ds + out->n_roles + out->n_revroles;
+  if (ts.joint) e->rd_last_changed = out->n_ds + out->n_roles + out->n_revroles;  // (sizes lwse_ds_resident_tick's publish grid)
   e->last_changed[1] = out->n_place;
   if (slot_out) *slot_out = slot;
   return LWSE_OK;
@@ -2034,6 +2097,8 @@ LWSE_API int lwse_resident_tick_wait(lwse_engine* e, lwse_tick* t) {
   if (!e || !t) return LWSE_ERR_INVALID_ARG;
   std::lock_guard<std::mutex> lock(e->mu);
   if (!e->r_loaded) return LWSE_ERR_NOT_READY;
+  // a joint tick at the head of the ring stays in flight: only lwse_joint_tick_wait reports its DS lists
+  if (e->t_submitted != e->t_waited && e->tslot[e->t_waited & 1u].joint) return LWSE_ERR_INVALID_ARG;
   DeviceGuard guard(e->device);
   TickCounts c;
   uint32_t slot = 0;
@@ -2161,6 +2226,63 @@ LWSE_API int lwse_sweep_ds_host(lwse_engine* e, const lwse_ds_tables* h) {
 // ---------------------------------------------------------------------------
 // Resident DisaggregatedSet tables
 // ---------------------------------------------------------------------------
+// Enqueue the resident DS sweep of tick slot `slot` on `s` (pdl: programmatically dependent on the kernel
+// before it, the patch scatter; the sweep waits at its top).  pl[0..2] receive the
+// slot's three lists for the publish kernel; pl[0].count + 3 is the slot's publish ticket.
+static int enqueue_ds_sweep(lwse_engine* e, uint32_t slot, bool first, cudaStream_t s, bool pdl, lwse::PublishListHost* pl,
+                            int* launched_out) {
+  uint8_t* chg_v = static_cast<uint8_t*>(e->rd_chg_dev.p) + slot * e->rd_chg_bytes;
+  uint8_t* chg_d = static_cast<uint8_t*>(e->rd_chg.d) + slot * e->rd_chg_bytes;
+  uint32_t* cnt = static_cast<uint32_t*>(e->rd_counts.p) + slot * 16u;
+  lwse_ds_tables d{};
+  d.ds = (const lwse_ds_rec*)e->rd_ds.p;
+  d.n_ds = e->rdn_ds;
+  d.roles = (const lwse_ds_role_rec*)e->rd_roles.p;
+  d.n_roles = e->rdn_roles;
+  d.revroles = (const lwse_ds_revrole_rec*)e->rd_revroles.p;
+  d.n_revroles = e->rdn_revroles;
+  lwse::DsResidentArgs r{};
+  r.ds_committed = (lwse_ds_out*)e->rd_ds_out.p;
+  r.role_committed = (lwse_ds_role_out*)e->rd_role_out.p;
+  r.revrole_committed = (lwse_ds_revrole_out*)e->rd_revrole_out.p;
+  r.role_scratch = (lwse_ds_role_out*)e->rd_role_scratch.p;
+  r.revrole_scratch = (lwse_ds_revrole_out*)e->rd_revrole_scratch.p;
+  r.ds_rows = reinterpret_cast<uint32_t*>(chg_v + e->rd_chg_off[0]);
+  r.ds_outs = reinterpret_cast<lwse_ds_out*>(chg_v + e->rd_chg_off[1]);
+  r.role_rows = reinterpret_cast<uint32_t*>(chg_v + e->rd_chg_off[2]);
+  r.role_outs = reinterpret_cast<lwse_ds_role_out*>(chg_v + e->rd_chg_off[3]);
+  r.revrole_rows = reinterpret_cast<uint32_t*>(chg_v + e->rd_chg_off[4]);
+  r.revrole_outs = reinterpret_cast<lwse_ds_revrole_out*>(chg_v + e->rd_chg_off[5]);
+  r.counts = cnt;
+  r.first = first ? 1u : 0u;
+  int cuda_err = 0;
+  const int launched = lwse::launch_ds_resident_sweep(&d, &r, e->sm_count, s, pdl, &cuda_err);
+  if (launched < 0) return fail_cuda(e, (cudaError_t)cuda_err);
+  e->launches += (uint64_t)launched;
+  *launched_out = launched;
+  pl[0] = {r.ds_rows, r.ds_outs, reinterpret_cast<uint32_t*>(chg_d + e->rd_chg_off[0]), chg_d + e->rd_chg_off[1], cnt + 0, e->rdn_ds,
+           (uint32_t)sizeof(lwse_ds_out)};
+  pl[1] = {r.role_rows, r.role_outs, reinterpret_cast<uint32_t*>(chg_d + e->rd_chg_off[2]), chg_d + e->rd_chg_off[3], cnt + 1,
+           e->rdn_roles, (uint32_t)sizeof(lwse_ds_role_out)};
+  pl[2] = {r.revrole_rows, r.revrole_outs, reinterpret_cast<uint32_t*>(chg_d + e->rd_chg_off[4]), chg_d + e->rd_chg_off[5], cnt + 2,
+           e->rdn_revroles, (uint32_t)sizeof(lwse_ds_revrole_out)};
+  return LWSE_OK;
+}
+
+static void fill_ds_tick_outputs(const lwse_engine* e, uint32_t slot, uint32_t n_ds, uint32_t n_roles, uint32_t n_revroles,
+                                 lwse_ds_tick* t) {
+  const uint8_t* base = static_cast<const uint8_t*>(e->rd_chg.h) + slot * e->rd_chg_bytes;
+  t->n_ds = n_ds < e->rdn_ds ? n_ds : e->rdn_ds;
+  t->n_roles = n_roles < e->rdn_roles ? n_roles : e->rdn_roles;
+  t->n_revroles = n_revroles < e->rdn_revroles ? n_revroles : e->rdn_revroles;
+  t->ds_rows = reinterpret_cast<const uint32_t*>(base + e->rd_chg_off[0]);
+  t->ds_out = reinterpret_cast<const lwse_ds_out*>(base + e->rd_chg_off[1]);
+  t->role_rows = reinterpret_cast<const uint32_t*>(base + e->rd_chg_off[2]);
+  t->role_out = reinterpret_cast<const lwse_ds_role_out*>(base + e->rd_chg_off[3]);
+  t->revrole_rows = reinterpret_cast<const uint32_t*>(base + e->rd_chg_off[4]);
+  t->revrole_out = reinterpret_cast<const lwse_ds_revrole_out*>(base + e->rd_chg_off[5]);
+}
+
 LWSE_API int lwse_ds_resident_load(lwse_engine* e, const lwse_ds_tables* h) {
   if (!e || !h) return LWSE_ERR_INVALID_ARG;
   if ((h->n_ds && !h->ds) || (h->n_roles && !h->roles) || (h->n_revroles && !h->revroles)) return LWSE_ERR_INVALID_ARG;
@@ -2172,6 +2294,7 @@ LWSE_API int lwse_ds_resident_load(lwse_engine* e, const lwse_ds_tables* h) {
   }
   cudaStream_t s = e->stream;
   LWSE_CUDA(e, cudaStreamSynchronize(s));  // (the previous DS tick's publish kernel is done with the lists)
+  LWSE_CUDA(e, cudaStreamSynchronize(e->pub_stream));  // (so is a joint tick's)
   e->rd_loaded = false;
   const size_t b_ds = (size_t)h->n_ds * sizeof(lwse_ds_rec), b_ro = (size_t)h->n_roles * sizeof(lwse_ds_role_rec),
                b_rr = (size_t)h->n_revroles * sizeof(lwse_ds_revrole_rec);
@@ -2191,11 +2314,19 @@ LWSE_API int lwse_ds_resident_load(lwse_engine* e, const lwse_ds_tables* h) {
     e->rd_chg_off[k] = off;
     off += align256(sizes[k] + 16);
   }
-  LWSE_CUDA(e, e->rd_chg_dev.reserve(off));
-  LWSE_CUDA(e, e->rd_chg.reserve(off));
-  LWSE_CUDA(e, e->rd_counts.reserve(64));
+  e->rd_chg_bytes = off;
+  LWSE_CUDA(e, e->rd_chg_dev.reserve(2 * off));  // two tick slots (joint ticks in flight)
+  LWSE_CUDA(e, e->rd_chg.reserve(2 * off));
+  LWSE_CUDA(e, e->rd_counts.reserve(128));
   LWSE_CUDA(e, e->rd_tickw.reserve(64));
-  LWSE_CUDA(e, cudaMemsetAsync(e->rd_counts.p, 0, 64, s));
+  LWSE_CUDA(e, cudaMemsetAsync(e->rd_counts.p, 0, 128, s));
+  // the ring's tick words and per-slot counters (publish ticket): a DS-only joint tick uses them on an
+  // engine that never called lwse_resident_load (which resets the counters itself)
+  if (!e->r_counts.p) {
+    LWSE_CUDA(e, e->r_counts.reserve(128));
+    LWSE_CUDA(e, cudaMemsetAsync(e->r_counts.p, 0, 128, s));
+  }
+  LWSE_CUDA(e, e->tickw.reserve(256));
   if (b_ds) LWSE_CUDA(e, cudaMemcpyAsync(e->rd_ds.p, h->ds, b_ds, cudaMemcpyHostToDevice, s));
   if (b_ro) LWSE_CUDA(e, cudaMemcpyAsync(e->rd_roles.p, h->roles, b_ro, cudaMemcpyHostToDevice, s));
   if (b_rr) LWSE_CUDA(e, cudaMemcpyAsync(e->rd_revroles.p, h->revroles, b_rr, cudaMemcpyHostToDevice, s));
@@ -2221,48 +2352,18 @@ LWSE_API int lwse_ds_resident_tick(lwse_engine* e, lwse_ds_tick* t) {
   if (rc != LWSE_OK) return rc;
   cudaStream_t s = e->stream;
   bool wrote = false;
-  rc = apply_patches_locked(e, t->segs, t->n_segs, &wrote, 0xFFFFFFFFu, s, 0, nullptr, 0, nullptr, false, /*ds=*/true);
+  rc = apply_patches_locked(e, t->segs, t->n_segs, &wrote, 0xFFFFFFFFu, s, 0, nullptr, 0, nullptr, false, kDsTableIds);
   if (rc != LWSE_OK) return rc;
-  uint8_t* chg_v = static_cast<uint8_t*>(e->rd_chg_dev.p);
-  uint8_t* chg_d = static_cast<uint8_t*>(e->rd_chg.d);
-  uint32_t* cnt = static_cast<uint32_t*>(e->rd_counts.p);
-  lwse_ds_tables d{};
-  d.ds = (const lwse_ds_rec*)e->rd_ds.p;
-  d.n_ds = e->rdn_ds;
-  d.roles = (const lwse_ds_role_rec*)e->rd_roles.p;
-  d.n_roles = e->rdn_roles;
-  d.revroles = (const lwse_ds_revrole_rec*)e->rd_revroles.p;
-  d.n_revroles = e->rdn_revroles;
-  lwse::DsResidentArgs r{};
-  r.ds_committed = (lwse_ds_out*)e->rd_ds_out.p;
-  r.role_committed = (lwse_ds_role_out*)e->rd_role_out.p;
-  r.revrole_committed = (lwse_ds_revrole_out*)e->rd_revrole_out.p;
-  r.role_scratch = (lwse_ds_role_out*)e->rd_role_scratch.p;
-  r.revrole_scratch = (lwse_ds_revrole_out*)e->rd_revrole_scratch.p;
-  r.ds_rows = reinterpret_cast<uint32_t*>(chg_v + e->rd_chg_off[0]);
-  r.ds_outs = reinterpret_cast<lwse_ds_out*>(chg_v + e->rd_chg_off[1]);
-  r.role_rows = reinterpret_cast<uint32_t*>(chg_v + e->rd_chg_off[2]);
-  r.role_outs = reinterpret_cast<lwse_ds_role_out*>(chg_v + e->rd_chg_off[3]);
-  r.revrole_rows = reinterpret_cast<uint32_t*>(chg_v + e->rd_chg_off[4]);
-  r.revrole_outs = reinterpret_cast<lwse_ds_revrole_out*>(chg_v + e->rd_chg_off[5]);
-  r.counts = cnt;
-  r.first = e->rd_first ? 1u : 0u;
-  int cuda_err = 0;
+  lwse::PublishListHost pl[3];
   // behind the scatter kernel: programmatically dependent, the sweep waits at its top
-  int launched = lwse::launch_ds_resident_sweep(&d, &r, e->sm_count, s, wrote, &cuda_err);
-  if (launched < 0) return fail_cuda(e, (cudaError_t)cuda_err);
-  e->launches += (uint64_t)launched;
-  lwse::PublishListHost pl[3] = {
-      {r.ds_rows, r.ds_outs, reinterpret_cast<uint32_t*>(chg_d + e->rd_chg_off[0]), chg_d + e->rd_chg_off[1], cnt + 0, e->rdn_ds,
-       (uint32_t)sizeof(lwse_ds_out)},
-      {r.role_rows, r.role_outs, reinterpret_cast<uint32_t*>(chg_d + e->rd_chg_off[2]), chg_d + e->rd_chg_off[3], cnt + 1,
-       e->rdn_roles, (uint32_t)sizeof(lwse_ds_role_out)},
-      {r.revrole_rows, r.revrole_outs, reinterpret_cast<uint32_t*>(chg_d + e->rd_chg_off[4]), chg_d + e->rd_chg_off[5], cnt + 2,
-       e->rdn_revroles, (uint32_t)sizeof(lwse_ds_revrole_out)}};
+  int launched = 0;
+  rc = enqueue_ds_sweep(e, 0, e->rd_first, s, wrote, pl, &launched);
+  if (rc != LWSE_OK) return rc;
   uint32_t seq = ++e->rd_seq;
   if (seq == 0) seq = ++e->rd_seq;
-  launched = lwse::launch_publish(pl, nullptr, static_cast<uint32_t*>(e->rd_tickw.d), 4, seq, cnt + 3, e->rd_last_changed, s,
-                                  &cuda_err, nullptr, 0, /*pdl=*/launched > 0);
+  int cuda_err = 0;
+  launched = lwse::launch_publish(pl, nullptr, static_cast<uint32_t*>(e->rd_tickw.d), 4, seq, pl[0].count + 3, e->rd_last_changed,
+                                  s, &cuda_err, nullptr, 0, /*pdl=*/launched > 0);
   if (launched < 0) return fail_cuda(e, (cudaError_t)cuda_err);
   e->launches += (uint64_t)launched;
   volatile uint32_t* hw = static_cast<volatile uint32_t*>(e->rd_tickw.h);
@@ -2271,16 +2372,7 @@ LWSE_API int lwse_ds_resident_tick(lwse_engine* e, lwse_ds_tick* t) {
     const cudaError_t a = cudaStreamSynchronize(s);
     return fail_cuda(e, werr != cudaSuccess ? werr : a != cudaSuccess ? a : cudaErrorUnknown);
   }
-  const uint8_t* base = static_cast<const uint8_t*>(e->rd_chg.h);
-  t->n_ds = hw[0] < e->rdn_ds ? hw[0] : e->rdn_ds;
-  t->n_roles = hw[1] < e->rdn_roles ? hw[1] : e->rdn_roles;
-  t->n_revroles = hw[2] < e->rdn_revroles ? hw[2] : e->rdn_revroles;
-  t->ds_rows = reinterpret_cast<const uint32_t*>(base + e->rd_chg_off[0]);
-  t->ds_out = reinterpret_cast<const lwse_ds_out*>(base + e->rd_chg_off[1]);
-  t->role_rows = reinterpret_cast<const uint32_t*>(base + e->rd_chg_off[2]);
-  t->role_out = reinterpret_cast<const lwse_ds_role_out*>(base + e->rd_chg_off[3]);
-  t->revrole_rows = reinterpret_cast<const uint32_t*>(base + e->rd_chg_off[4]);
-  t->revrole_out = reinterpret_cast<const lwse_ds_revrole_out*>(base + e->rd_chg_off[5]);
+  fill_ds_tick_outputs(e, 0, hw[0], hw[1], hw[2], t);
   e->rd_last_changed = t->n_ds + t->n_roles + t->n_revroles;
   e->rd_first = false;
   return LWSE_OK;
@@ -2305,6 +2397,85 @@ LWSE_API int lwse_ds_resident_outputs(lwse_engine* e, lwse_ds_out* ds_out, lwse_
                                  cudaMemcpyDeviceToHost, s));
   LWSE_CUDA(e, cudaStreamSynchronize(s));
   return LWSE_OK;
+}
+
+// ---------------------------------------------------------------------------
+// Joint LWS + DS tick
+// ---------------------------------------------------------------------------
+// One part's segments, checked as the scatter would check them, before anything is enqueued: a refused
+// joint tick changes nothing.
+static int check_joint_part(lwse_engine* e, const lwse_patch_seg* segs, uint32_t n_segs, uint32_t ids) {
+  if (n_segs > LWSE_TICK_MAX_SEGS || (n_segs && !segs)) return LWSE_ERR_INVALID_ARG;
+  for (uint32_t i = 0; i < n_segs; i++) {
+    const lwse_patch_seg& g = segs[i];
+    void* base;
+    uint64_t rows;
+    uint32_t rb;
+    if (!resident_table(e, g.table, &base, &rows, &rb, ids)) return LWSE_ERR_INVALID_ARG;
+    if (g.n == 0) continue;
+    if (!g.values || (!(g.flags & LWSE_PATCH_RANGE) && !g.rows)) return LWSE_ERR_INVALID_ARG;
+    if ((g.flags & LWSE_PATCH_RANGE) && (uint64_t)g.first_row + g.n > rows) return LWSE_ERR_BAD_TABLE;
+  }
+  return LWSE_OK;
+}
+
+static int joint_submit_locked(lwse_engine* e, const lwse_tick* lws, const lwse_ds_tick* ds) {
+  if (!e->rd_loaded || (lws && !e->r_loaded) || (lws && (lws->flags & LWSE_TICK_PLACE) && !e->r_place_loaded))
+    return LWSE_ERR_NOT_READY;
+  if (ds->flags != 0 || (lws && (lws->flags & LWSE_TICK_SHARED_OCCUPANCY))) return LWSE_ERR_INVALID_ARG;
+  int rc = lws ? check_joint_part(e, lws->segs, lws->n_segs, kLwsTableIds) : LWSE_OK;
+  if (rc == LWSE_OK) rc = check_joint_part(e, ds->segs, ds->n_segs, kDsTableIds);
+  if (rc != LWSE_OK) return rc;
+  if (e->t_submitted - e->t_waited >= 2) return LWSE_ERR_NOT_READY;
+  lwse_patch_seg segs[2 * LWSE_TICK_MAX_SEGS];
+  uint32_t n = 0;
+  for (uint32_t i = 0; lws && i < lws->n_segs; i++) segs[n++] = lws->segs[i];
+  for (uint32_t i = 0; i < ds->n_segs; i++) segs[n++] = ds->segs[i];
+  return tick_submit_locked(e, segs, n, lws ? lws->flags : LWSE_TICK_NO_SWEEP, /*joint=*/true);
+}
+
+static int joint_wait_locked(lwse_engine* e, lwse_tick* lws, lwse_ds_tick* ds) {
+  if (e->t_submitted == e->t_waited) return LWSE_ERR_NOT_READY;
+  const bool joint = e->tslot[e->t_waited & 1u].joint;
+  TickCounts c;
+  uint32_t slot = 0;
+  const int rc = tick_wait_locked(e, &c, &slot);
+  if (rc != LWSE_OK) return rc;
+  if (lws) fill_tick_outputs(e, slot, c, lws);
+  if (joint) {
+    fill_ds_tick_outputs(e, slot, c.n_ds, c.n_roles, c.n_revroles, ds);
+  } else {  // an LWS tick: no DS lists
+    ds->ds_rows = ds->role_rows = ds->revrole_rows = nullptr;
+    ds->ds_out = nullptr;
+    ds->role_out = nullptr;
+    ds->revrole_out = nullptr;
+    ds->n_ds = ds->n_roles = ds->n_revroles = 0;
+  }
+  return LWSE_OK;
+}
+
+LWSE_API int lwse_joint_tick_submit(lwse_engine* e, const lwse_tick* lws, const lwse_ds_tick* ds) {
+  if (!e || !ds) return LWSE_ERR_INVALID_ARG;
+  std::lock_guard<std::mutex> lock(e->mu);
+  DeviceGuard guard(e->device);
+  return joint_submit_locked(e, lws, ds);
+}
+
+LWSE_API int lwse_joint_tick_wait(lwse_engine* e, lwse_tick* lws, lwse_ds_tick* ds) {
+  if (!e || !ds) return LWSE_ERR_INVALID_ARG;
+  std::lock_guard<std::mutex> lock(e->mu);
+  DeviceGuard guard(e->device);
+  return joint_wait_locked(e, lws, ds);
+}
+
+LWSE_API int lwse_joint_tick(lwse_engine* e, lwse_tick* lws, lwse_ds_tick* ds) {
+  if (!e || !ds) return LWSE_ERR_INVALID_ARG;
+  std::lock_guard<std::mutex> lock(e->mu);
+  DeviceGuard guard(e->device);
+  if (e->t_submitted != e->t_waited) return LWSE_ERR_NOT_READY;  // the ticks in flight keep their results for _wait
+  int rc = joint_submit_locked(e, lws, ds);
+  if (rc == LWSE_OK) rc = joint_wait_locked(e, lws, ds);
+  return rc;
 }
 
 // ---------------------------------------------------------------------------

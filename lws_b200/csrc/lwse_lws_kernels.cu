@@ -1135,9 +1135,9 @@ int launch_lws_sweep(const lwse_lws_tables* t, const lwse_node_rec* d_nodes, uin
 // tick: change lists to the host
 // --------------------------------------------------------------------------
 // The last kernel of a tick (lwse_resident_tick).  The sweep / placement kernels appended the
-// changed rows to device-memory lists; this kernel copies the used part of up to three lists into
-// pinned, mapped host memory with coalesced stores and then raises the sequence word the host
-// spins on — no stream synchronize, no copy-engine launch on the critical path.
+// changed rows to device-memory lists; this kernel copies the used part of up to three lists (six for
+// a joint LWS + DS tick) into pinned, mapped host memory with coalesced stores and then raises the
+// sequence word the host spins on — no stream synchronize, no copy-engine launch on the critical path.
 // Ordering: a system-scope fence costs microseconds and fences from many threads queue up behind
 // each other (one per writing thread measured 15-25 us for this kernel), so there is exactly ONE.
 // Usual case, one CTA: bar.sync, then thread 0 writes the counts, fences at system scope (cumulative:
@@ -1154,10 +1154,13 @@ struct PublishList {
   uint32_t out_vec;     // uint4 per result row (rows of 16-byte multiples), else 0
   uint32_t out_words;   // 32-bit words per result row of rows narrower than 16 bytes, else 0
 };
+// kLists = 3: one controller's lists (an LWS tick: LWS, group, placement; a DS tick: DS, role,
+// revision-role).  kLists = 6: a joint tick, the LWS tick's three lists then the DS tick's three.
+template <int kLists>
 struct PublishArgs {
-  PublishList list[3];
+  PublishList list[kLists];
   const uint32_t* extra;   // nullable: one more device word to publish (the placement round counter)
-  uint32_t* host_words;    // mapped host: [k] = count of list k, [3] = extra, then the sequence word at [seq_slot]
+  uint32_t* host_words;    // mapped host: count of list k at [host_word(k)], [3] = extra, the sequence word at [seq_slot]
   uint32_t seq_slot;
   uint32_t seq;
   uint32_t* ticket;
@@ -1169,16 +1172,21 @@ struct PublishArgs {
 
 constexpr uint32_t kPublishThreads = 1024;
 
-__global__ void __launch_bounds__(kPublishThreads) publish_lists_kernel(const PublishArgs a) {
+// Host word of list k's count: lists 0-2 at [0..2] (then [3] extra, [4] the sequence word of a tick
+// slot), lists 3-5 at [5..7].
+__host__ __device__ constexpr uint32_t host_word(uint32_t k) { return k < 3u ? k : k + 2u; }
+
+template <int kLists>
+__global__ void __launch_bounds__(kPublishThreads) publish_lists_kernel(const PublishArgs<kLists> a) {
   __shared__ uint32_t s_last;
   pdl_wait_prior();  // every producer kernel of the tick has completed: lists and counters are final
   const uint32_t gtid = blockIdx.x * blockDim.x + threadIdx.x, gsize = gridDim.x * blockDim.x;
   // the counts and each thread's first elements are requested together (the lists' memory is valid
   // up to the capacity): one L2 round trip instead of two before the first store leaves
-  uint32_t counts[3] = {0, 0, 0}, row0[3] = {0, 0, 0};
-  uint4 out0[3];
+  uint32_t counts[kLists] = {}, row0[kLists] = {};
+  uint4 out0[kLists];
 #pragma unroll
-  for (uint32_t k = 0; k < 3; k++) {
+  for (uint32_t k = 0; k < kLists; k++) {
     const PublishList& l = a.list[k];
     out0[k] = make_uint4(0, 0, 0, 0);
     if (l.count == nullptr) continue;
@@ -1187,7 +1195,7 @@ __global__ void __launch_bounds__(kPublishThreads) publish_lists_kernel(const Pu
     if (gtid < l.capacity * l.out_vec) out0[k] = __ldcg(l.src_outs + gtid);
   }
 #pragma unroll
-  for (uint32_t k = 0; k < 3; k++) {
+  for (uint32_t k = 0; k < kLists; k++) {
     const PublishList& l = a.list[k];
     if (l.count == nullptr) continue;
     const uint32_t n = min(counts[k], l.capacity);
@@ -1214,9 +1222,9 @@ __global__ void __launch_bounds__(kPublishThreads) publish_lists_kernel(const Pu
   if (last && threadIdx.x == 0) {
     volatile uint32_t* hw = a.host_words;
 #pragma unroll
-    for (uint32_t k = 0; k < 3; k++) {
+    for (uint32_t k = 0; k < kLists; k++) {
       if (a.list[k].count == nullptr) continue;
-      hw[k] = counts[k];
+      hw[host_word(k)] = counts[k];
       *a.list[k].count = 0u;  // ready for the next tick (stream-ordered)
     }
     if (a.extra != nullptr) hw[3] = __ldcg(a.extra);
@@ -1239,13 +1247,13 @@ struct PublishListHost {
   uint32_t out_bytes;
 };
 
-// lists[0..2]: the three slots (host_words[k] receives the count of slot k).
-int launch_publish(const PublishListHost* lists, const uint32_t* d_extra, uint32_t* h_words, uint32_t seq_slot,
-                   uint32_t seq, uint32_t* d_ticket, uint32_t expected_rows, cudaStream_t s, int* cuda_err,
-                   uint32_t* d_clear, uint32_t n_clear, bool pdl) {
+template <int kLists>
+static int launch_publish_lists(const PublishListHost* lists, const uint32_t* d_extra, uint32_t* h_words, uint32_t seq_slot,
+                                uint32_t seq, uint32_t* d_ticket, uint32_t expected_rows, cudaStream_t s, int* cuda_err,
+                                uint32_t* d_clear, uint32_t n_clear, bool pdl) {
   *cuda_err = 0;
-  PublishArgs a{};
-  for (int k = 0; k < 3; k++) {
+  PublishArgs<kLists> a{};
+  for (int k = 0; k < kLists; k++) {
     const bool vec = lists[k].out_bytes % 16u == 0;
     a.list[k] = PublishList{lists[k].src_rows, static_cast<const uint4*>(lists[k].src_outs), lists[k].dst_rows,
                             static_cast<uint4*>(lists[k].dst_outs), lists[k].count, lists[k].capacity,
@@ -1266,12 +1274,28 @@ int launch_publish(const PublishListHost* lists, const uint32_t* d_extra, uint32
   // ONE CTA for the usual few thousand rows (no ticket stage then); more when the previous tick reported many
   unsigned grid = expected_rows / 8192u + 1u;
   if (grid > 32u) grid = 32u;
-  const cudaError_t e = launch_pdl(publish_lists_kernel, dim3(grid), dim3(kPublishThreads), 0, s, g_pdl && pdl, a);
+  const cudaError_t e = launch_pdl(publish_lists_kernel<kLists>, dim3(grid), dim3(kPublishThreads), 0, s, g_pdl && pdl, a);
   if (e != cudaSuccess) {
     *cuda_err = (int)e;
     return -1;
   }
   return 1;
+}
+
+// lists[0..2]: the three slots (host_words[k] receives the count of slot k).
+int launch_publish(const PublishListHost* lists, const uint32_t* d_extra, uint32_t* h_words, uint32_t seq_slot,
+                   uint32_t seq, uint32_t* d_ticket, uint32_t expected_rows, cudaStream_t s, int* cuda_err,
+                   uint32_t* d_clear, uint32_t n_clear, bool pdl) {
+  return launch_publish_lists<3>(lists, d_extra, h_words, seq_slot, seq, d_ticket, expected_rows, s, cuda_err, d_clear, n_clear,
+                                 pdl);
+}
+
+// A joint tick: lists[0..5], counts to host_words[0..2] and [5..7] (host_word).
+int launch_publish_joint(const PublishListHost* lists, const uint32_t* d_extra, uint32_t* h_words, uint32_t seq_slot,
+                         uint32_t seq, uint32_t* d_ticket, uint32_t expected_rows, cudaStream_t s, int* cuda_err,
+                         uint32_t* d_clear, uint32_t n_clear) {
+  return launch_publish_lists<6>(lists, d_extra, h_words, seq_slot, seq, d_ticket, expected_rows, s, cuda_err, d_clear, n_clear,
+                                 false);
 }
 
 // --------------------------------------------------------------------------
@@ -1474,7 +1498,8 @@ cudaError_t set_sweep_carveout(int pct) {
   set((const void*)lws_sweep_kernel<32>);
   set((const void*)scatter_rows_kernel);
   set((const void*)scatter_rows_desc_kernel);
-  set((const void*)publish_lists_kernel);
+  set((const void*)publish_lists_kernel<3>);
+  set((const void*)publish_lists_kernel<6>);
   return e;
 }
 

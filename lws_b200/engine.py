@@ -25,6 +25,7 @@ SYMBOLS = {
     "lwse_abi_version": ([], C.c_uint32),
     "lwse_stream": ([C.c_void_p], C.c_void_p),
     "lwse_launch_count": ([C.c_void_p], C.c_uint64),
+    "lwse_graph_tick_count": ([C.c_void_p], C.c_uint64),
     "lwse_shard_of": ([C.c_uint64, C.c_uint32], C.c_uint32),
     "lwse_hash64": ([C.c_void_p, C.c_size_t], C.c_uint64),
     "lwse_upload_nodes": ([C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32], C.c_int),
@@ -84,6 +85,9 @@ SYMBOLS = {
     "lwse_ds_resident_load": ([C.c_void_p, C.POINTER(R.DsTables)], C.c_int),
     "lwse_ds_resident_tick": ([C.c_void_p, C.POINTER(R.DsTick)], C.c_int),
     "lwse_ds_resident_outputs": ([C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p], C.c_int),
+    "lwse_joint_tick": ([C.c_void_p, C.POINTER(R.Tick), C.POINTER(R.DsTick)], C.c_int),
+    "lwse_joint_tick_submit": ([C.c_void_p, C.POINTER(R.Tick), C.POINTER(R.DsTick)], C.c_int),
+    "lwse_joint_tick_wait": ([C.c_void_p, C.POINTER(R.Tick), C.POINTER(R.DsTick)], C.c_int),
     "lwse_group_keys_host": ([C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p], C.c_int),
     "lwse_subgroup_keys_host": (
         [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p], C.c_int),
@@ -165,6 +169,11 @@ class Engine:
     @property
     def launch_count(self) -> int:
         return lib().lwse_launch_count(self._h)
+
+    @property
+    def graph_tick_count(self) -> int:
+        """Resident ticks replayed as one CUDA graph since creation."""
+        return lib().lwse_graph_tick_count(self._h)
 
     # ------------------------------------------------------------------ nodes
     def upload_nodes(self, nodes: np.ndarray, n_domains: int):
@@ -485,7 +494,10 @@ class Engine:
         """One DS tick: patches in, listed result rows out → dict of numpy views of engine-owned
         pinned memory (valid until the next resident call)."""
         self._check(lib().lwse_ds_resident_tick(self._h, C.byref(tick)))
+        return self._ds_tick_views(tick)
 
+    @staticmethod
+    def _ds_tick_views(tick: "R.DsTick"):
         def view(ptr, n, dtype):
             if not ptr or n == 0:
                 return np.zeros(0, dtype=dtype)
@@ -507,6 +519,25 @@ class Engine:
         o = (R.aligned_empty(n_ds, R.DS_OUT), R.aligned_empty(n_ro, R.DS_ROLE_OUT), R.aligned_empty(n_rr, R.DS_REVROLE_OUT))
         self._check(lib().lwse_ds_resident_outputs(self._h, *(R.ptr(x) for x in o)))
         return o
+
+    # ------------------------------------------------------------- joint tick
+    def joint_tick(self, tick, ds_tick):
+        """One tick of both controllers (``tick`` may be None: DS only) → (lws_result, ds_result), the
+        dicts of ``resident_tick`` and ``ds_resident_tick`` (lws_result None without ``tick``)."""
+        self._check(lib().lwse_joint_tick(self._h, C.byref(tick) if tick is not None else None, C.byref(ds_tick)))
+        return (self._tick_views(tick) if tick is not None else None), self._ds_tick_views(ds_tick)
+
+    def joint_tick_submit(self, tick, ds_tick):
+        """Enqueue a joint tick and return; it shares the two-slot ring of ``resident_tick_submit``."""
+        self._check(lib().lwse_joint_tick_submit(self._h, C.byref(tick) if tick is not None else None, C.byref(ds_tick)))
+
+    def joint_tick_wait(self):
+        """Wait for the OLDEST tick in flight, joint or LWS-only → (lws_result, ds_result); an LWS-only
+        tick reports no DS rows.  lws_result is None on an engine without resident LWS tables."""
+        tick = R.Tick() if hasattr(self, "_resident_shape") else None
+        ds_tick = R.DsTick()
+        self._check(lib().lwse_joint_tick_wait(self._h, C.byref(tick) if tick is not None else None, C.byref(ds_tick)))
+        return (self._tick_views(tick) if tick is not None else None), self._ds_tick_views(ds_tick)
 
     # ------------------------------------------------------------- group keys
     def group_keys_host(self, strings) -> np.ndarray:
